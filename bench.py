@@ -4,8 +4,11 @@ bench.py -- entity-steps/s of the batched rollout + collision path (BASELINE.jso
 
     python bench.py --gpus N --steps K --warmup W            # B200 engine
     python bench.py --impl reference --steps K --warmup W     # CPU arm (oracle port, all cores)
+    python bench.py --steps K --warmup W --dump-outputs DIR  # + the results of the last timed step as .npy
 
-A "step" is one full rollout (reset + T ticks) of this rank's batch of synthetic scenarios.
+A "step" is one full rollout (reset + T ticks) of this rank's batch of synthetic scenarios.  Every
+timed region of the headline workload runs K steps; the sub-records run --sub-steps.  The inputs are
+seeded, so two runs with the same arguments roll out the same scenarios and actions.
 
 Headline workload = BASELINE.json configs[2] per-GPU shard (C3): 12 500 scenarios x 64
 VehicleController entities x 256 ticks of dt = 0.1 with random accel/steer actions,
@@ -40,6 +43,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the source tree (which may be read-only)
 REPO = os.path.dirname(os.path.abspath(__file__))
 if REPO not in sys.path:
     sys.path.insert(0, REPO)
@@ -76,6 +80,9 @@ def parse_args():
     ap.add_argument("--actions", default="rng", choices=["rng", "table"],
                     help="action source of the headline value for c3 / c5 (the other one is reported beside it)")
     ap.add_argument("--sub-steps", type=int, default=5)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline workload computed as DIR/<name>.npy "
+                         "(rank 0's batch)")
     return ap.parse_args()
 
 
@@ -335,6 +342,55 @@ def _worker_step(_):
     return steps, time.perf_counter() - t0
 
 
+def result_fields(wl: Workload):
+    """The state fields a rollout of `wl` computes: (discrete per scenario, discrete per entity,
+    continuous per scenario, continuous per entity)."""
+    disc_n = ("tick", "done", "first_coll_tick", "first_coll_pair", "n_pair_ticks", "rss_flags", "t")
+    disc_nm = ("present", "collided") + (("rss_state", "rss_last") if wl.rss else ())
+    cont_n = ("ego_avg_speed", "ego_max_speed", "ego_dist")
+    cont_nm = ("pose", "vel", "dist", "speed") + (("safe_dist", "safe_ratio") if wl.rss else ()) + \
+        (("force",) if wl.name == "c4" else ())
+    if wl.name == "c4":
+        disc_nm += ("goal_idx",)
+    return disc_n, disc_nm, cont_n, cont_nm
+
+
+DUMP_ENTITIES = 1 << 16  # per-entity planes of at most this many entities are written (~13 MB)
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(wl: Workload, eng, out_dir: str) -> None:
+    """
+    Write what the last rollout of `eng` computed as out_dir/<name>.npy (float64), so that two builds can be
+    compared output for output: every per-scenario field over the whole batch, and the per-entity planes
+    and ego collision events (rows: scenario, tick, slot, t) of a fixed, seeded sample of scenarios
+    (`sample_scenarios`; the full planes of C3 take ~100 MB).  Per-entity planes keep the engine's layout,
+    restricted to the sampled scenarios' slots.  Every value written is finite.
+    """
+    disc_n, disc_nm, cont_n, cont_nm = result_fields(wl)
+    n = min(wl.N, max(1, DUMP_ENTITIES // wl.M))
+    sample = np.sort(np.random.default_rng(0).choice(wl.N, n, replace=False))
+    cols = (sample[:, None] * wl.M + np.arange(wl.M)).ravel()
+    out = {"sample_scenarios": sample}
+    out.update({k: eng.get(k) for k in disc_n + cont_n})
+    out.update({k: eng.get(k)[..., cols] for k in disc_nm + cont_nm})
+    ev = eng.events()
+    ev = ev[np.isin(ev["scenario"], sample)]
+    out["events"] = np.stack([ev[f].astype(np.float64) for f in ("scenario", "tick", "slot", "t")], axis=1)
+    if "safe_ratio" in out:  # no hazard: the ratio is +inf (as in the reference); written as 0, flagged in safe_ratio_inf
+        inf = np.isposinf(out["safe_ratio"])
+        out["safe_ratio_inf"] = inf
+        out["safe_ratio"] = np.where(inf, 0.0, out["safe_ratio"])
+    out = {k: np.ascontiguousarray(v, np.float64) for k, v in out.items()}
+    bad = [k for k, v in out.items() if not np.isfinite(v).all()]
+    assert not bad, f"--dump-outputs: non-finite values in {bad}"
+    total = sum(v.nbytes for v in out.values())
+    assert total <= DUMP_LIMIT, f"--dump-outputs would write {total} bytes"
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def oracle_parity_and_baseline(wl: Workload, gpu, budget_s: float = 10.0, n_min: int = 4, n_max: int = 2048):
     """
     Roll the first n scenarios of this rank's batch out on the CPU oracle (one core, ~budget_s of work),
@@ -344,6 +400,7 @@ def oracle_parity_and_baseline(wl: Workload, gpu, budget_s: float = 10.0, n_min:
     from oracle.runner import OracleEngine
 
     n_min = {"c2": 23, "c4": 1, "c5": 2}.get(wl.name, n_min)
+    disc_n, disc_nm, cont_n, cont_nm = result_fields(wl)
     n = min(n_min, wl.N)
     while True:
         scene, actions = wl.oracle_sample(n)
@@ -368,13 +425,6 @@ def oracle_parity_and_baseline(wl: Workload, gpu, budget_s: float = 10.0, n_min:
     }
     # ---- parity: GPU rows of the same scenarios
     sl = slice(0, n * M)
-    disc_n = ("tick", "done", "first_coll_tick", "first_coll_pair", "n_pair_ticks", "rss_flags", "t")
-    disc_nm = ("present", "collided") + (("rss_state", "rss_last") if wl.rss else ())
-    cont_n = ("ego_avg_speed", "ego_max_speed", "ego_dist")
-    cont_nm = ("pose", "vel", "dist", "speed") + (("safe_dist", "safe_ratio") if wl.rss else ()) + \
-        (("force",) if wl.name == "c4" else ())
-    if wl.name == "c4":
-        disc_nm += ("goal_idx",)
     mism, max_err = [], 0.0
     for k in disc_n:
         if not np.array_equal(gpu.get(k)[:n], eng.get(k), equal_nan=True):
@@ -579,21 +629,13 @@ class Bench:
 
         for _ in range(max(1, min(warmup, 2))):
             e2e_step()
-        # (a step of a few ms -- C2 -- is timed over enough steps to fill ~60 ms of wall clock: five of them are
-        # within the jitter of the host thread that enqueues a few dozen copies and launches per step)
-        for attempt in range(2):
-            self.barrier()
-            t0 = time.perf_counter()
-            for _ in range(steps):
-                e2e_step()
-            self.torch.cuda.synchronize(self.dev)
-            wall = time.perf_counter() - t0
-            self.launches += 2 * steps
-            short = self.allreduce(1.0 if wall < 0.03 else 0.0, "MAX") > 0.0
-            if attempt == 1 or not short:
-                break
-            steps = int(min(64, max(steps + 1, np.ceil(steps * 0.06 / max(wall, 1e-4)))))
-            steps = int(self.allreduce(float(steps), "MAX"))
+        self.barrier()
+        t0 = time.perf_counter()
+        for _ in range(steps):
+            e2e_step()
+        self.torch.cuda.synchronize(self.dev)
+        wall = time.perf_counter() - t0
+        self.launches += 2 * steps
         # the host-buffer path must reproduce the resident path bit for bit
         for k, v in ref.items():
             got = hr.results[k].numpy()
@@ -634,6 +676,8 @@ class Bench:
         elapsed_ms, kern_ms, reset_ms, clocks = self.time_device(eng, source(primary), steps, warmup)
         ticks = eng.get("tick")
         assert np.array_equal(ticks, wl.expected_ticks), "every scenario must run its full number of ticks"
+        if headline and args.dump_outputs and self.rank == 0:
+            dump_outputs(wl, eng, args.dump_outputs)
         total_steps = self.allreduce(float(wl.steps_expected), "SUM")
         value = total_steps * steps / (elapsed_ms / 1e3)
         ref = {k: eng.get(k).copy() for k in ("ego_avg_speed", "ego_max_speed", "ego_dist", "first_coll_tick",
@@ -677,16 +721,16 @@ class Bench:
             out["e2e"] = self.time_e2e(wl, eng, primary, steps, warmup, ref)
         if has_actions and headline:  # the other action source beside it
             other = "table" if primary == "rng" else "rng"
-            e2, k2, _, _ = self.time_device(eng, source(other), max(3, steps // 2), 2)
+            e2, k2, _, _ = self.time_device(eng, source(other), steps, 2)
             for k, v in ref.items():
                 assert np.array_equal(eng.get(k), v, equal_nan=True), f"{other} action source: {k} differs"
-            rec = {"value": total_steps * max(3, steps // 2) / (e2 / 1e3), "kernel_ms": k2, "action_source": other,
+            rec = {"value": total_steps * steps / (e2 / 1e3), "kernel_ms": k2, "action_source": other,
                    "bit_equal_to_headline": True}
             if not args.no_e2e:
                 table_dev = None  # free the resident table before the e2e buffers are allocated
-                rec["e2e"] = self.time_e2e(wl, eng, other, max(3, steps // 2), 2, ref)
+                rec["e2e"] = self.time_e2e(wl, eng, other, steps, 2, ref)
                 if other == "table":
-                    r32 = self.time_e2e(wl, eng, "table_f32", max(3, steps // 2), 2, {"tick": ref["tick"]})
+                    r32 = self.time_e2e(wl, eng, "table_f32", steps, 2, {"tick": ref["tick"]})
                     rec["e2e_fp32_table"] = r32
             out["table_path" if other == "table" else "rng_path"] = rec
         del eng
