@@ -45,7 +45,7 @@
 extern "C" {
 #endif
 
-#define SG_ABI_VERSION 12
+#define SG_ABI_VERSION 13
 
 /* entity slot kinds (who produces the slot's next pose each tick) */
 enum SgKind {
@@ -310,9 +310,42 @@ typedef struct SgInputs {
   SgActionRng rng;
 } SgInputs;
 
+/* Closed-loop environment (sg_env_observe / sg_env_reward): which slots a policy drives, what it
+   observes and how it is rewarded.  Agent a of scenario n is slot agent_slot[n*A + a] (-1: padding).
+   An observation row has F = 4 + 3*L + 10*K + (road ? 2 : 0) floats, all in the agent's frame
+   (x, y, h its pose, (c, s) = (cos h, sin h), rot(dx, dy) = (c*dx + s*dy, -s*dx + c*dy)):
+     self       speed (controller state), rot(vx, vy), vel[3] (heading rate)
+     target     per lookahead tau: q = position_at_t(own trajectory, t + tau, clamped):
+                rot(qx - x, qy - y), remainder(qh - h, 2 pi)
+     neighbours the K present other slots j with the smallest (d2, j), d2 = dx*dx + dy*dy < radius^2
+                (radius <= 0: no cut-off), ascending: rot(dx, dy), cos(hj - h), sin(hj - h),
+                rot(vxj - vx, vyj - vy), width_j, length_j, [etype_j == pedestrian], 1; missing: zeros
+     road       driveable surface strictly contains (x, y); distance from (x, y) to the surface's rings
+                (zeros when the network has no driveable area)
+   Absent / padding agents get zero rows.  Reward terms (after a tick, against the snapshot the last
+   observe took): progress = dist - dist_snap; collision = collided rose 0 -> 1; off_road = network has
+   driveable area and the present slot is not strictly inside it; tracking = -|(x, y) - position_at_t(own
+   trajectory, t, clamped)[:2]|; rss = the slot is the ego and rss_flags gained a bit.  Absent / padding
+   agents get zero terms.  reward = sum_k w[k] * term_k. */
+typedef struct SgEnvSpec {
+  int32_t n_agents;          /* A >= 1 */
+  int32_t k_neighbours;      /* K, 0..32 */
+  const int32_t* agent_slot; /* [N*A] device */
+  double radius;
+  int32_t n_lookahead;       /* L, 0..8 */
+  int32_t road;              /* non-zero: append the road block */
+  double lookahead[8];       /* seconds */
+  double weights[5];         /* progress, collision, off_road, tracking, rss */
+  /* snapshot written by sg_env_observe for the scenarios it observes, read by sg_env_reward (device) */
+  double* snap_dist;         /* [N*A] */
+  uint8_t* snap_collided;    /* [N*A] */
+  int64_t* snap_pair_ticks;  /* [N] */
+  uint8_t* snap_rss;         /* [N] */
+} SgEnvSpec;
+
 int sg_abi_version(void);
 /* sizeof() of the ABI structs so bindings can verify their mirror: which = 0 SgParams,
-   1 SgScene, 2 SgState, 3 SgInputs, 4 SgEvent, 5 SgActionRng, 6 SgHostResults */
+   1 SgScene, 2 SgState, 3 SgInputs, 4 SgEvent, 5 SgActionRng, 6 SgHostResults, 7 SgEnvSpec */
 int64_t sg_sizeof(int which);
 const char* sg_last_error(void);
 void sg_default_params(SgParams* p);
@@ -320,6 +353,28 @@ void sg_default_params(SgParams* p);
 /* State.reset(t0) + Metric.reset + Agent.reset: state/state.py:106-143,
    scenario_gym.py:217-225, controller.py:100-103, metrics/trajectory.py:13-18 */
 int sg_reset(const SgScene* scene, const SgParams* params, SgState* state, int device, void* stream);
+
+/* sg_reset of the scenarios with mask[n] != 0 only (mask [N], device memory; NULL: all of them).  Every
+   field of every other scenario is left as it was, and event_count is not touched. */
+int sg_reset_scenarios(const SgScene* scene, const SgParams* params, SgState* state, const uint8_t* mask,
+                       int device, void* stream);
+
+/* Observations of the agents of SgEnvSpec (see there) for the scenarios with mask[n] != 0 (NULL: all):
+   obs [N][A][F] fp32 (computed in fp64, rounded once), agent_mask [N][A] (the slot exists and is present),
+   and the snapshot the next sg_env_reward compares against.  Rows of other scenarios are not written. */
+int sg_env_observe(const SgScene* scene, const SgParams* params, const SgState* state, const SgEnvSpec* spec,
+                   const uint8_t* mask, float* obs, uint8_t* agent_mask, int device, void* stream);
+
+/* Rewards of one environment step, after the tick and before any reset: reward [N][A], terms [N][A][5]
+   (fp32).  For the scenarios whose done flag is set (an environment steps only scenarios that are not
+   done, so: the ones this tick finished) terminated [N] = a collision / ego_collision / ego_off_road
+   condition of params->terminal holds at this tick, truncated [N] = otherwise (max_length); both are 0
+   for the other scenarios.  The conditions are recomputed from the state as the tick decided them:
+   collision = n_pair_ticks grew since the snapshot, ego_collision = collided[first_slot],
+   ego_off_road = first_slot absent or not strictly inside the driveable surface. */
+int sg_env_reward(const SgScene* scene, const SgParams* params, const SgState* state, const SgEnvSpec* spec,
+                  float* reward, float* terms, uint8_t* terminated, uint8_t* truncated, int device,
+                  void* stream);
 
 /* n_ticks x ScenarioGym.step() fused on device (scenario_gym.py:227-254): agents /
    batch replay -> State.step -> RSSDistances -> terminal check -> metrics.  Scenarios

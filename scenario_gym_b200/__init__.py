@@ -8,12 +8,13 @@ gym / engine does (there is no CPU fallback).
 """
 from .actions import FixedTAction, ScenarioAction, UpdateStateVariableAction, UserDefinedAction
 from .entity import BoundingBox, CatalogEntry, Entity, MiscObject, Pedestrian, Vehicle
+from .env import ObsSpec, VecScenarioEnv
 from .gym import ScenarioGym
 from .plugins import (RSS, Action, ActionTableAgent, Agent, CollisionMetric, CollisionObservation,
                       CombinedSensor, Controller, GlobalCollisionDetector, combine_observations,
                       EgoAvgSpeed, EgoDistanceTravelled, EgoLocalizationSensor, EgoMaxSpeed,
                       FutureCollisionDetector, FutureCollisionObservation, Metric,
-                      Observation, PedestrianAction, PedestrianAgent, PIDAgent, PIDController, ReplayTrajectoryAgent,
+                      Observation, PedestrianAction, PedestrianAgent, PIDAgent, PIDController, PolicyAgent, ReplayTrajectoryAgent,
                       ReplayTrajectoryController, RSSDistances, RSSParameters, Sensor,
                       SingleEntityObservation, SocialForce, SocialForceParameters, StateCallback,
                       TeleportAction, VehicleAction, VehicleController, cache_mean, cache_metric,

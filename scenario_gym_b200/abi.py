@@ -11,7 +11,7 @@ import math
 import os
 from typing import Dict, Optional
 
-ABI_VERSION = 12
+ABI_VERSION = 13
 
 # SgKind
 KIND_EMPTY, KIND_REPLAY, KIND_AGENT_REPLAY, KIND_VEHICLE, KIND_PEDESTRIAN, KIND_HOST, KIND_PID = range(7)
@@ -215,6 +215,32 @@ class SgHostResults(C.Structure):
     ]
 
 
+class SgEnvSpec(C.Structure):
+    _fields_ = [
+        ("n_agents", C.c_int32),
+        ("k_neighbours", C.c_int32),
+        ("agent_slot", _p),
+        ("radius", C.c_double),
+        ("n_lookahead", C.c_int32),
+        ("road", C.c_int32),
+        ("lookahead", C.c_double * 8),
+        ("weights", C.c_double * 5),
+        ("snap_dist", _p),
+        ("snap_collided", _p),
+        ("snap_pair_ticks", _p),
+        ("snap_rss", _p),
+    ]
+
+
+# number of reward terms of sg_env_reward: progress, collision, off_road, tracking, rss
+ENV_TERMS = ("progress", "collision", "off_road", "tracking", "rss")
+
+
+def env_n_features(k_neighbours: int, n_lookahead: int, road: bool) -> int:
+    """Floats per observation row of sg_env_observe (include/sg_b200.h, SgEnvSpec)."""
+    return 4 + 3 * n_lookahead + 10 * k_neighbours + (2 if road else 0)
+
+
 # (field, dtype, shape spec) of every SgState array; shape tokens: N, M, NM, W, E, T
 STATE_FIELDS = [
     ("pose", "float64", ("6", "NM")),
@@ -299,7 +325,7 @@ def default_params() -> SgParams:
 EXPORTS = [
     "abi_version", "sizeof", "last_error", "default_params", "reset", "rollout",
     "test_box_pairs", "future_collisions", "fill_random_actions", "rollout_host", "host_h2d_bytes",
-    "host_d2h_bytes",
+    "host_d2h_bytes", "reset_scenarios", "env_observe", "env_reward",
 ]
 
 
@@ -324,6 +350,16 @@ def bind(lib: C.CDLL, prefix: str) -> Dict[str, object]:
     get("last_error", C.c_char_p, [])
     get("default_params", None, [C.POINTER(SgParams)])
     get("reset", C.c_int, [C.POINTER(SgScene), C.POINTER(SgParams), C.POINTER(SgState), C.c_int, _p])
+    # the closed-loop environment's entry points: the product exports them (tests/test_abi.py checks every
+    # declared symbol); of the CPU oracle's libraries only libsg_env_oracle.so does (oracle/env_runner.py)
+    get("reset_scenarios", C.c_int,
+        [C.POINTER(SgScene), C.POINTER(SgParams), C.POINTER(SgState), _p, C.c_int, _p], required=False)
+    get("env_observe", C.c_int,
+        [C.POINTER(SgScene), C.POINTER(SgParams), C.POINTER(SgState), C.POINTER(SgEnvSpec), _p, _p, _p,
+         C.c_int, _p], required=False)
+    get("env_reward", C.c_int,
+        [C.POINTER(SgScene), C.POINTER(SgParams), C.POINTER(SgState), C.POINTER(SgEnvSpec), _p, _p, _p, _p,
+         C.c_int, _p], required=False)
     get("rollout", C.c_int,
         [C.POINTER(SgScene), C.POINTER(SgParams), C.POINTER(SgState), C.POINTER(SgInputs),
          C.c_int, C.c_int, _p])
@@ -347,7 +383,10 @@ def bind(lib: C.CDLL, prefix: str) -> Dict[str, object]:
 
     if f["abi_version"]() != ABI_VERSION:
         raise RuntimeError(f"ABI version mismatch: lib {f['abi_version']()} != {ABI_VERSION}")
-    for which, st in enumerate((SgParams, SgScene, SgState, SgInputs, SgEvent, SgActionRng, SgHostResults)):
+    structs = [SgParams, SgScene, SgState, SgInputs, SgEvent, SgActionRng, SgHostResults]
+    if "env_observe" in f:  # (a library that takes SgEnvSpec knows its size)
+        structs.append(SgEnvSpec)
+    for which, st in enumerate(structs):
         if f["sizeof"](which) != C.sizeof(st):
             raise RuntimeError(
                 f"ABI struct {st.__name__}: lib {f['sizeof'](which)} B != ctypes {C.sizeof(st)} B"

@@ -44,7 +44,7 @@ static int check_rng(const SgActionRng& r) {
 }
 
 static int launch(const SgScene* sc, const SgParams* p, SgState* st, const SgInputs* in, int n_ticks,
-                  int device, void* stream, int reset) {
+                  int device, void* stream, int reset, const uint8_t* reset_mask = nullptr) {
   if (!sc || !p || !st) return set_msg("null argument");
   if (sc->n_slots < 1 || sc->n_slots > 1024) return set_msg("n_slots must be in 1..1024");
   if (sc->n_scenarios < 1) return set_msg("n_scenarios must be >= 1");
@@ -79,7 +79,7 @@ static int launch(const SgScene* sc, const SgParams* p, SgState* st, const SgInp
   if (smem > 227 * 1024) return set_msg("scenario does not fit in shared memory");
   cudaStream_t s = (cudaStream_t)stream;
   if (reset) {
-    err = sgi_launch_reset(rss, big, blocks, threads, smem, s, *sc, *p, *st, L);
+    err = sgi_launch_reset(rss, big, blocks, threads, smem, s, *sc, *p, *st, L, reset_mask);
     if (err != cudaSuccess) return set_err("sg_reset_kernel launch", err);
     return 0;
   }
@@ -142,6 +142,7 @@ int64_t sg_sizeof(int which) {
     case 4: return sizeof(SgEvent);
     case 5: return sizeof(SgActionRng);
     case 6: return sizeof(SgHostResults);
+    case 7: return sizeof(SgEnvSpec);
   }
   return -1;
 }
@@ -194,6 +195,59 @@ int sg_reset(const SgScene* scene, const SgParams* params, SgState* state, int d
 int sg_rollout(const SgScene* scene, const SgParams* params, SgState* state, const SgInputs* inputs,
                int n_ticks, int device, void* stream) {
   return launch(scene, params, state, inputs, n_ticks, device, stream, 0);
+}
+
+int sg_reset_scenarios(const SgScene* scene, const SgParams* params, SgState* state, const uint8_t* mask,
+                       int device, void* stream) {
+  return launch(scene, params, state, nullptr, 0, device, stream, 1, mask);
+}
+
+// the checks sg_env_observe and sg_env_reward share; `view` gets the scene with its plane stride stated
+static int check_env(const SgScene* sc, const SgParams* p, const SgState* st, const SgEnvSpec* e, SgScene* view) {
+  if (!sc || !p || !st || !e) return set_msg("null argument");
+  if (sc->n_slots < 1 || sc->n_slots > 1024) return set_msg("n_slots must be in 1..1024");
+  if (sc->n_scenarios < 1) return set_msg("n_scenarios must be >= 1");
+  if (sc->plane_stride > 0) return set_msg("sg_env_*: scenario windows are not supported");
+  if (e->n_agents < 1 || e->n_agents > sc->n_slots) return set_msg("SgEnvSpec.n_agents must be in 1..n_slots");
+  if (e->k_neighbours < 0 || e->k_neighbours > 32) return set_msg("SgEnvSpec.k_neighbours must be in 0..32");
+  if (e->n_lookahead < 0 || e->n_lookahead > 8) return set_msg("SgEnvSpec.n_lookahead must be in 0..8");
+  for (int k = 0; k < e->n_lookahead; ++k)
+    if (!isfinite(e->lookahead[k])) return set_msg("SgEnvSpec.lookahead must be finite");
+  if (!isfinite(e->radius)) return set_msg("SgEnvSpec.radius must be finite");
+  if (!e->agent_slot || !e->snap_dist || !e->snap_collided || !e->snap_pair_ticks || !e->snap_rss)
+    return set_msg("SgEnvSpec: agent_slot / snapshot buffers missing");
+  *view = *sc;
+  view->plane_stride = (int64_t)sc->n_scenarios * sc->n_slots;
+  view->scenario_base = 0;
+  return 0;
+}
+
+int sg_env_observe(const SgScene* scene, const SgParams* params, const SgState* state, const SgEnvSpec* spec,
+                   const uint8_t* mask, float* obs, uint8_t* agent_mask, int device, void* stream) {
+  SgScene view;
+  int rc = check_env(scene, params, state, spec, &view);
+  if (rc) return rc;
+  if (!obs || !agent_mask) return set_msg("null argument");
+  cudaError_t err = cudaSetDevice(device);
+  if (err != cudaSuccess) return set_err("cudaSetDevice", err);
+  err = sgi_launch_env_observe((cudaStream_t)stream, view, *state, *spec, mask, obs, agent_mask);
+  if (err != cudaSuccess) return set_err("sg_env_observe_kernel launch", err);
+  return 0;
+}
+
+int sg_env_reward(const SgScene* scene, const SgParams* params, const SgState* state, const SgEnvSpec* spec,
+                  float* reward, float* terms, uint8_t* terminated, uint8_t* truncated, int device,
+                  void* stream) {
+  SgScene view;
+  int rc = check_env(scene, params, state, spec, &view);
+  if (rc) return rc;
+  if (!reward || !terms || !terminated || !truncated) return set_msg("null argument");
+  cudaError_t err = cudaSetDevice(device);
+  if (err != cudaSuccess) return set_err("cudaSetDevice", err);
+  err = sgi_launch_env_reward((cudaStream_t)stream, view, *params, *state, *spec, reward, terms, terminated,
+                              truncated);
+  if (err != cudaSuccess) return set_err("sg_env_reward_kernel launch", err);
+  return 0;
 }
 
 int sg_fill_random_actions(const SgActionRng* rng, int tick0, int n_ticks, int64_t nm, double* out,

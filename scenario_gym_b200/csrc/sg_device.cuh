@@ -359,16 +359,12 @@ static __device__ __noinline__ bool surface_contains(const SgScene sc, int n, in
   return false;
 }
 
-// shapely.ops.nearest_points(surface, Point(px, py))[0]: the point itself when it lies in the
-// (closed) surface, else the closest point on a ring (GEOS LineSegment::closestPoint: projection
-// factor r = ((p - a).(b - a)) / |b - a|^2, the projection for 0 < r < 1, else the closer end point)
-static __device__ __noinline__ double2 surface_nearest(const SgScene sc, int n, int k, double px, double py) {
+// The closest point to (px, py) on the rings of polygons [q0, q1) (GEOS LineSegment::closestPoint:
+// projection factor r = ((p - a).(b - a)) / |b - a|^2, the projection for 0 < r < 1, else the closer end
+// point); best_d2 gets its squared distance.  No ring: (px, py) and INFINITY.
+SG_DEV double2 ring_nearest(const SgScene& sc, int64_t q0, int64_t q1, double px, double py, double& best_d2) {
   double2 best = make_double2(px, py);
-  const int r = sc.rn_of[n];
-  const int64_t q0 = sc.rn_poly_off[3 * r + k], q1 = sc.rn_poly_off[3 * r + k + 1];
-  for (int64_t q = q0; q < q1; ++q)
-    if (polygon_side(sc.rn_edges, sc.rn_edge_off[q], sc.rn_edge_off[q + 1], px, py) >= 0) return best;
-  double best_d2 = INFINITY;
+  best_d2 = INFINITY;
   for (int64_t e = sc.rn_edge_off[q0]; e < sc.rn_edge_off[q1]; ++e) {
     const double ax = __ldg(sc.rn_edges + 4 * e), ay = __ldg(sc.rn_edges + 4 * e + 1);
     const double bx = __ldg(sc.rn_edges + 4 * e + 2), by = __ldg(sc.rn_edges + 4 * e + 3);
@@ -387,6 +383,18 @@ static __device__ __noinline__ double2 surface_nearest(const SgScene sc, int n, 
     if (d2 < best_d2) { best_d2 = d2; best = make_double2(cx, cy); }
   }
   return best;
+}
+
+// shapely.ops.nearest_points(surface, Point(px, py))[0]: the point itself when it lies in the
+// (closed) surface, else the closest point on a ring
+static __device__ __noinline__ double2 surface_nearest(const SgScene sc, int n, int k, double px, double py) {
+  const int r = sc.rn_of[n];
+  const int64_t q0 = sc.rn_poly_off[3 * r + k], q1 = sc.rn_poly_off[3 * r + k + 1];
+  for (int64_t q = q0; q < q1; ++q)
+    if (polygon_side(sc.rn_edges, sc.rn_edge_off[q], sc.rn_edge_off[q + 1], px, py) >= 0)
+      return make_double2(px, py);
+  double d2;
+  return ring_nearest(sc, q0, q1, px, py, d2);
 }
 
 // SocialForce._force_boundary (pedestrian/social_force.py:190-211) for surface k

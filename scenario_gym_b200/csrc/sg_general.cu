@@ -354,10 +354,11 @@ sg_rollout_kernel(SgScene sc, SgParams p, SgState st, SgInputs in, int n_ticks, 
 }
 
 // State.reset(t0) + Agent/Metric/StateCallback resets (reference state/state.py:106-143,
-// controller.py:100-103, metrics/trajectory.py:13-18, metrics/rss/callback.py:44-55)
+// controller.py:100-103, metrics/trajectory.py:13-18, metrics/rss/callback.py:44-55).
+// mask != NULL: only the scenarios with mask[n] != 0 (a whole group leaves, so its barriers stay matched)
 template <bool RSS, int MAXT>
 __global__ void __launch_bounds__(MAXT, MAXT >= 1024 ? 1 : 2)
-sg_reset_kernel(SgScene sc, SgParams p, SgState st, GroupLayout L) {
+sg_reset_kernel(SgScene sc, SgParams p, SgState st, GroupLayout L, const uint8_t* __restrict__ mask) {
   extern __shared__ __align__(16) unsigned char smem[];
   const int G = L.G, M = sc.n_slots, W = L.W;
   const int gpb = blockDim.x / G;
@@ -365,6 +366,7 @@ sg_reset_kernel(SgScene sc, SgParams p, SgState st, GroupLayout L) {
   const int s = threadIdx.x - gl * G;
   const int n = blockIdx.x * gpb + gl;
   if (gl >= gpb || n >= sc.n_scenarios) return;
+  if (mask && !mask[n]) return;
   Grp c;
   setup_group(c, sc, L, smem, gl, s, n);
   c.sorted = 0;  // no broad phase at reset
@@ -462,13 +464,13 @@ sg_reset_kernel(SgScene sc, SgParams p, SgState st, GroupLayout L) {
 template <bool RSS>
 static cudaError_t launch_reset_t(bool big, int blocks, int threads, size_t smem, cudaStream_t s,
                                 const SgScene& sc, const SgParams& p, const SgState& st,
-                                const GroupLayout& L) {
+                                const GroupLayout& L, const uint8_t* mask) {
   auto kern = big ? sg_reset_kernel<RSS, 1024> : sg_reset_kernel<RSS, SG_THREADS>;
   if (smem > 48 * 1024) {
     cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (err != cudaSuccess) return err;
   }
-  kern<<<blocks, threads, smem, s>>>(sc, p, st, L);
+  kern<<<blocks, threads, smem, s>>>(sc, p, st, L, mask);
   return cudaGetLastError();
 }
 
@@ -486,9 +488,10 @@ static cudaError_t launch_rollout_t(bool big, int blocks, int threads, size_t sm
 }
 
 cudaError_t sgi_launch_reset(bool rss, bool big, int blocks, int threads, size_t smem, cudaStream_t s,
-                             const SgScene& sc, const SgParams& p, const SgState& st, const GroupLayout& L) {
-  return rss ? launch_reset_t<true>(big, blocks, threads, smem, s, sc, p, st, L)
-             : launch_reset_t<false>(big, blocks, threads, smem, s, sc, p, st, L);
+                             const SgScene& sc, const SgParams& p, const SgState& st, const GroupLayout& L,
+                             const uint8_t* mask) {
+  return rss ? launch_reset_t<true>(big, blocks, threads, smem, s, sc, p, st, L, mask)
+             : launch_reset_t<false>(big, blocks, threads, smem, s, sc, p, st, L, mask);
 }
 
 cudaError_t sgi_launch_rollout(bool ped, bool rss, bool big, int blocks, int threads, size_t smem,

@@ -7,8 +7,10 @@
 #include "sg_layout.h"
 #include "sg_pcg.cuh"
 
+// mask: [N] scenarios to reset (NULL: all)
 cudaError_t sgi_launch_reset(bool rss, bool big, int blocks, int threads, size_t smem, cudaStream_t s,
-                             const SgScene& sc, const SgParams& p, const SgState& st, const GroupLayout& L);
+                             const SgScene& sc, const SgParams& p, const SgState& st, const GroupLayout& L,
+                             const uint8_t* mask);
 cudaError_t sgi_launch_rollout(bool ped, bool rss, bool big, int blocks, int threads, size_t smem,
                                cudaStream_t s, const SgScene& sc, const SgParams& p, const SgState& st,
                                const SgInputs& in, const SgRngDev& rng, int n_ticks, const GroupLayout& L);
@@ -43,5 +45,11 @@ cudaError_t sgi_launch_radius(cudaStream_t s, const SgState& st, int n_scen, int
                               const double* r, uint8_t* out);
 // rows: an upper bound of the union rows of the scene's scenarios (a window holds fewer than n_union_rows)
 cudaError_t sgi_launch_union(cudaStream_t s, const SgScene& sc, int64_t rows);
+// closed-loop environment (sg_env.cu); `sc` has its plane stride stated
+cudaError_t sgi_launch_env_observe(cudaStream_t s, const SgScene& sc, const SgState& st, const SgEnvSpec& e,
+                                   const uint8_t* mask, float* obs, uint8_t* agent_mask);
+cudaError_t sgi_launch_env_reward(cudaStream_t s, const SgScene& sc, const SgParams& p, const SgState& st,
+                                  const SgEnvSpec& e, float* reward, float* terms, uint8_t* terminated,
+                                  uint8_t* truncated);
 cudaError_t sgi_launch_traj(cudaStream_t s, const double* rows, int K, const double* t, int64_t n, int mode,
                             double* pos, uint8_t* ok, double* vel);

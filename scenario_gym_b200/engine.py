@@ -111,10 +111,41 @@ class Engine:
         return int(sum(t.numel() * t.element_size() for t in self._state_t.values()))
 
     # ------------------------------------------------------------------ API
-    def reset(self) -> None:
-        """State.reset + metric/controller resets for every scenario (sg_reset)."""
-        self._check(self.lib["reset"](C.byref(self._sc), C.byref(self.params), C.byref(self._st),
-                                      self.dev_index, self._stream()))
+    def reset(self, mask: Optional[torch.Tensor] = None) -> None:
+        """
+        State.reset + metric/controller resets for every scenario (sg_reset), or -- ``mask``: a uint8 / bool
+        device tensor [N] -- for the scenarios with ``mask[n] != 0`` only (sg_reset_scenarios; the other
+        scenarios and the event count are left as they are).
+        """
+        if mask is None:
+            self._check(self.lib["reset"](C.byref(self._sc), C.byref(self.params), C.byref(self._st),
+                                          self.dev_index, self._stream()))
+            return
+        m = self._scenario_mask(mask)
+        self._check(self.lib["reset_scenarios"](C.byref(self._sc), C.byref(self.params), C.byref(self._st),
+                                                m.data_ptr(), self.dev_index, self._stream()))
+
+    def _scenario_mask(self, mask: torch.Tensor) -> torch.Tensor:
+        if not isinstance(mask, torch.Tensor) or mask.device != self.device or mask.numel() != self.N \
+                or mask.dtype not in (torch.uint8, torch.bool):
+            raise ValueError(f"mask must be a uint8 / bool tensor of {self.N} entries on {self.device}")
+        return mask.contiguous().view(torch.uint8) if mask.dtype == torch.bool else mask.contiguous()
+
+    def env_observe(self, spec: abi.SgEnvSpec, obs: torch.Tensor, agent_mask: torch.Tensor,
+                    mask: Optional[torch.Tensor] = None) -> None:
+        """sg_env_observe into preallocated ``obs`` (fp32 [N, A, F]) / ``agent_mask`` (uint8 [N, A])."""
+        m = None if mask is None else self._scenario_mask(mask)
+        self._check(self.lib["env_observe"](C.byref(self._sc), C.byref(self.params), C.byref(self._st),
+                                            C.byref(spec), None if m is None else m.data_ptr(), obs.data_ptr(),
+                                            agent_mask.data_ptr(), self.dev_index, self._stream()))
+
+    def env_reward(self, spec: abi.SgEnvSpec, reward: torch.Tensor, terms: torch.Tensor,
+                   terminated: torch.Tensor, truncated: torch.Tensor) -> None:
+        """sg_env_reward into preallocated reward (fp32 [N, A]), terms (fp32 [N, A, 5]) and flags (uint8 [N])."""
+        self._check(self.lib["env_reward"](C.byref(self._sc), C.byref(self.params), C.byref(self._st),
+                                           C.byref(spec), reward.data_ptr(), terms.data_ptr(),
+                                           terminated.data_ptr(), truncated.data_ptr(), self.dev_index,
+                                           self._stream()))
 
     def build_union_on_device(self) -> torch.Tensor:
         """

@@ -9,6 +9,7 @@ Lowering: what ``create_agent`` returns decides each entity's device slot kind
   None                          -> batch replay            (entity/batch.py)
   ReplayTrajectoryAgent         -> clamped replay agent    (agent.py:118-128)
   ActionTableAgent              -> VehicleController, whole action table on device
+  PolicyAgent                   -> VehicleController on device, actions from VecScenarioEnv.step (env only)
   Agent + VehicleController     -> VehicleController on device, policy ``_step`` on the host per tick
   PedestrianAgent + SocialForce -> social force on device
   any other Agent               -> pose from ``agent.step(state)`` on the host per tick
@@ -27,7 +28,7 @@ from . import abi
 from .entity import Entity
 from .packing import ScenarioSpec, SlotSpec, pack_scenarios
 from .plugins import (ActionTableAgent, Agent, CollisionMetric, EgoLocalizationSensor, Metric,
-                      PedestrianAgent, PIDAgent, PIDController, RandomActionAgent, ReplayTrajectoryAgent, ReplayTrajectoryController, RSSDistances,
+                      PedestrianAgent, PIDAgent, PIDController, PolicyAgent, RandomActionAgent, ReplayTrajectoryAgent, ReplayTrajectoryController, RSSDistances,
                       SocialForce, StateCallback, VehicleAction, VehicleController, _create_agent,
                       _DeviceMetric)
 from .scenario import Scenario
@@ -157,8 +158,14 @@ class ScenarioGym:
             if isinstance(m, _DeviceMetric):
                 m._value = None
 
+    def _refuse_env_agents(self) -> None:
+        if getattr(self, "_any_env_policy", False):
+            raise RuntimeError("the batch has PolicyAgents, whose actions come from a policy: "
+                               "run it through VecScenarioEnv")
+
     def step(self) -> None:
         """One tick for every scenario that is not done (reference :227-254)."""
+        self._refuse_env_agents()
         self._sync_params()
         eng = self._engine
         N, M = eng.N, eng.M
@@ -225,6 +232,7 @@ class ScenarioGym:
         """Roll every scenario out to ``is_done`` (reference :256-267)."""
         if render:
             raise ValueError("rendering is out of scope of the device engine (no viewer)")
+        self._refuse_env_agents()
         self.reset_scenario()
         if self._host_mode:
             while not all(st.is_done for st in self.states):
@@ -319,6 +327,7 @@ class ScenarioGym:
 
         specs, self._slot_of, self._entity_of = [], [], []
         self._agent_kind: Dict[Agent, str] = {}
+        self._env_slots: List[List[int]] = [[] for _ in self.states]  # PolicyAgent slots per scenario
         veh_params, ped_params, pid_params = set(), set(), set()
         tables, random_agents = {}, {}
         for n, st in enumerate(self.states):
@@ -361,6 +370,9 @@ class ScenarioGym:
                     if type(agent) is ActionTableAgent:
                         self._agent_kind[agent] = "device"
                         tables[(n, s)] = agent.table
+                    elif type(agent) is PolicyAgent:
+                        self._agent_kind[agent] = "env_policy"
+                        self._env_slots[n].append(s)
                     elif type(agent) is RandomActionAgent:
                         self._agent_kind[agent] = "device"
                         random_agents[(n, s)] = agent
@@ -411,6 +423,7 @@ class ScenarioGym:
         kinds = set(self._agent_kind.values())
         self._any_host_policy = "host_policy" in kinds
         self._any_host_agent = "host" in kinds
+        self._any_env_policy = "env_policy" in kinds
         self._host_mode = bool(self._host_metric_protos or host_cbs or self._host_terminal
                                or self._any_host_policy or self._any_host_agent)
 

@@ -450,6 +450,20 @@ class RandomActionAgent(Agent):
         return VehicleAction(float(a[0]), float(a[1]))
 
 
+class PolicyAgent(Agent):
+    """
+    Vehicle agent whose VehicleActions come from the policy of a ``VecScenarioEnv``: the env scatters
+    each step's action tensor into the device's action rows, so the agent has no host-side ``_step``.
+    It runs only inside an env; ``ScenarioGym.step`` / ``rollout`` refuse a batch that contains one.
+    """
+
+    def __init__(self, entity: Entity, **controller_kwargs):
+        super().__init__(entity, VehicleController(entity, **controller_kwargs), EgoLocalizationSensor(entity))
+
+    def _step(self, observation) -> VehicleAction:
+        raise RuntimeError("PolicyAgent takes its actions from VecScenarioEnv.step()")
+
+
 def _create_agent(scenario, entity) -> Optional[Agent]:
     """Default: a replay agent for the entity named "ego" (reference agent.py:151-169)."""
     if entity.ref == "ego":
