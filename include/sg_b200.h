@@ -45,7 +45,7 @@
 extern "C" {
 #endif
 
-#define SG_ABI_VERSION 13
+#define SG_ABI_VERSION 14
 
 /* entity slot kinds (who produces the slot's next pose each tick) */
 enum SgKind {
@@ -312,7 +312,7 @@ typedef struct SgInputs {
 
 /* Closed-loop environment (sg_env_observe / sg_env_reward): which slots a policy drives, what it
    observes and how it is rewarded.  Agent a of scenario n is slot agent_slot[n*A + a] (-1: padding).
-   An observation row has F = 4 + 3*L + 10*K + (road ? 2 : 0) floats, all in the agent's frame
+   An observation row has F floats (below), all in the agent's frame
    (x, y, h its pose, (c, s) = (cos h, sin h), rot(dx, dy) = (c*dx + s*dy, -s*dx + c*dy)):
      self       speed (controller state), rot(vx, vy), vel[3] (heading rate)
      target     per lookahead tau: q = position_at_t(own trajectory, t + tau, clamped):
@@ -322,7 +322,24 @@ typedef struct SgInputs {
                 rot(vxj - vx, vyj - vy), width_j, length_j, [etype_j == pedestrian], 1; missing: zeros
      road       driveable surface strictly contains (x, y); distance from (x, y) to the surface's rings
                 (zeros when the network has no driveable area)
-   Absent / padding agents get zero rows.  Reward terms (after a tick, against the snapshot the last
+     lidar      (n_rays = R > 0) R readings, ray k along (ex, ey) = ray_dir[k] in the agent's frame, which must
+                be (cos, sin)(2 pi k / R) to within 1e-12 (the caller passes the values, so every
+                implementation uses the same bits).  World direction u = (c*ex - s*ey, s*ex + c*ey), ray
+                (x, y) + t*u, t >= 0.  Every present slot j != the agent's, of any type, is the oriented box
+                the collision test uses: (cj, sj) = (cos hj, sin hj), centre X = xj + (bcx*cj - bcy*sj),
+                Y = yj + (bcx*sj + bcy*cj), half extents hl = length / 2 along hj, hw = width / 2 across.
+                Hit test (closed set, slab form, this operation order, no FMA):
+                  p = (x - X, y - Y); ox = cj*px + sj*py, oy = -sj*px + cj*py;
+                  dx = cj*ux + sj*uy, dy = -sj*ux + cj*uy;
+                  per axis (o, d, e) in {(ox, dx, hl), (oy, dy, hw)}: d != 0: lo, hi = min, max of
+                  (-e - o) / d and (e - o) / d; d == 0: a miss if |o| > e, else (-inf, +inf);
+                  enter = max(lo_x, lo_y), exit = min(hi_x, hi_y); a hit iff exit >= enter and exit >= 0,
+                  at distance (enter > 0 ? enter : 0).
+                So a touching corner or a ray along an edge hits, an origin inside another box reads 0 and
+                boxes without width / size act as segments / points.  Reading = min(ray_range, smallest hit
+                distance over j) in fp64, rounded once to fp32 (ray_range when nothing is hit).
+   The row is F = 4 + 3*L + 10*K + (road ? 2 : 0) + R floats; with R = 0 it is the row without the lidar
+   block, bit for bit.  Absent / padding agents get zero rows.  Reward terms (after a tick, against the snapshot the last
    observe took): progress = dist - dist_snap; collision = collided rose 0 -> 1; off_road = network has
    driveable area and the present slot is not strictly inside it; tracking = -|(x, y) - position_at_t(own
    trajectory, t, clamped)[:2]|; rss = the slot is the ego and rss_flags gained a bit.  Absent / padding
@@ -341,6 +358,11 @@ typedef struct SgEnvSpec {
   uint8_t* snap_collided;    /* [N*A] */
   int64_t* snap_pair_ticks;  /* [N] */
   uint8_t* snap_rss;         /* [N] */
+  /* lidar block (appended after the road block; read by sg_env_observe only) */
+  int32_t n_rays;            /* R, 0..256 (0: no lidar block) */
+  int32_t _pad0;
+  double ray_range;          /* metres, finite and > 0 when R > 0 */
+  const double* ray_dir;     /* [R][2] device: unit directions in the agent frame (see above) */
 } SgEnvSpec;
 
 int sg_abi_version(void);

@@ -11,7 +11,7 @@ import math
 import os
 from typing import Dict, Optional
 
-ABI_VERSION = 13
+ABI_VERSION = 14
 
 # SgKind
 KIND_EMPTY, KIND_REPLAY, KIND_AGENT_REPLAY, KIND_VEHICLE, KIND_PEDESTRIAN, KIND_HOST, KIND_PID = range(7)
@@ -229,6 +229,10 @@ class SgEnvSpec(C.Structure):
         ("snap_collided", _p),
         ("snap_pair_ticks", _p),
         ("snap_rss", _p),
+        ("n_rays", C.c_int32),
+        ("_pad0", C.c_int32),
+        ("ray_range", C.c_double),
+        ("ray_dir", _p),
     ]
 
 
@@ -236,9 +240,17 @@ class SgEnvSpec(C.Structure):
 ENV_TERMS = ("progress", "collision", "off_road", "tracking", "rss")
 
 
-def env_n_features(k_neighbours: int, n_lookahead: int, road: bool) -> int:
+def env_n_features(k_neighbours: int, n_lookahead: int, road: bool, n_rays: int = 0) -> int:
     """Floats per observation row of sg_env_observe (include/sg_b200.h, SgEnvSpec)."""
-    return 4 + 3 * n_lookahead + 10 * k_neighbours + (2 if road else 0)
+    return 4 + 3 * n_lookahead + 10 * k_neighbours + (2 if road else 0) + n_rays
+
+
+def lidar_directions(n_rays: int):
+    """The [R, 2] fp64 ray directions of SgEnvSpec.ray_dir: (cos, sin)(2 pi k / R), numpy's values."""
+    import numpy as np
+
+    ang = 2.0 * np.pi * np.arange(n_rays) / n_rays
+    return np.ascontiguousarray(np.stack([np.cos(ang), np.sin(ang)], 1))
 
 
 # (field, dtype, shape spec) of every SgState array; shape tokens: N, M, NM, W, E, T

@@ -216,6 +216,12 @@ static int check_env(const SgScene* sc, const SgParams* p, const SgState* st, co
   if (!isfinite(e->radius)) return set_msg("SgEnvSpec.radius must be finite");
   if (!e->agent_slot || !e->snap_dist || !e->snap_collided || !e->snap_pair_ticks || !e->snap_rss)
     return set_msg("SgEnvSpec: agent_slot / snapshot buffers missing");
+  if (e->n_rays < 0 || e->n_rays > 256) return set_msg("SgEnvSpec.n_rays must be in 0..256");
+  if (e->n_rays > 0) {
+    if (!isfinite(e->ray_range) || !(e->ray_range > 0.0))
+      return set_msg("SgEnvSpec.ray_range must be finite and > 0 when n_rays > 0");
+    if (!e->ray_dir) return set_msg("SgEnvSpec.ray_dir missing (n_rays > 0)");
+  }
   *view = *sc;
   view->plane_stride = (int64_t)sc->n_scenarios * sc->n_slots;
   view->scenario_base = 0;

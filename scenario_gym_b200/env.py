@@ -8,6 +8,7 @@ is allocated once, when the env is built.
 """
 from __future__ import annotations
 
+import math
 from dataclasses import dataclass
 from typing import Callable, Dict, List, Mapping, Optional, Sequence, Tuple, Union
 
@@ -33,15 +34,20 @@ _FINAL_FIELDS = {"ego_avg_speed": "ego_avg_speed", "ego_max_speed": "ego_max_spe
 class ObsSpec:
     """What each agent observes (include/sg_b200.h, SgEnvSpec): ``k_neighbours`` (0..32) nearest present
     entities within ``radius`` metres (<= 0: no cut-off), its own trajectory ``lookahead`` seconds ahead
-    (at most 8 times) and, with ``road``, whether it is on the driveable surface and how far its edge is."""
+    (at most 8 times), with ``road`` whether it is on the driveable surface and how far its edge is, and with
+    ``lidar_rays`` = R (0..256) a planar lidar: R rays at angles 2 pi k / R from its heading, each reading the
+    distance to the first box of another present entity, at most ``lidar_range`` metres."""
     k_neighbours: int = 8
     radius: float = 50.0
     lookahead: Sequence[float] = (1.0, 2.0, 3.0)
     road: bool = False
+    lidar_rays: int = 0
+    lidar_range: float = 50.0
 
     @property
     def n_features(self) -> int:
-        return abi.env_n_features(int(self.k_neighbours), len(self.lookahead), bool(self.road))
+        return abi.env_n_features(int(self.k_neighbours), len(self.lookahead), bool(self.road),
+                                  int(self.lidar_rays))
 
 
 def _ego_policy(scenario: Scenario, entity: Entity):
@@ -84,6 +90,11 @@ class VecScenarioEnv:
         self.obs_spec = obs if obs is not None else ObsSpec()
         if not 0 <= int(self.obs_spec.k_neighbours) <= 32 or len(self.obs_spec.lookahead) > 8:
             raise ValueError("ObsSpec: k_neighbours must be in 0..32 and lookahead have at most 8 times")
+        R = int(self.obs_spec.lidar_rays)
+        if not 0 <= R <= 256:
+            raise ValueError(f"ObsSpec: lidar_rays must be in 0..256, got {self.obs_spec.lidar_rays}")
+        if R > 0 and not (math.isfinite(float(self.obs_spec.lidar_range)) and float(self.obs_spec.lidar_range) > 0):
+            raise ValueError(f"ObsSpec: lidar_range must be finite and > 0, got {self.obs_spec.lidar_range}")
         w = dict(DEFAULT_REWARD_WEIGHTS)
         if isinstance(reward_weights, Mapping):
             unknown = set(reward_weights) - set(abi.ENV_TERMS)
@@ -150,6 +161,11 @@ class VecScenarioEnv:
         for k, name in enumerate(abi.ENV_TERMS):
             spec.weights[k] = float(w[name])
         spec.agent_slot = self.agent_slots.data_ptr()
+        spec.n_rays, spec.ray_range = R, float(self.obs_spec.lidar_range)
+        # the lidar's ray directions, built once from numpy's values (the env keeps the tensor alive)
+        self._ray_dir = torch.from_numpy(abi.lidar_directions(R)).to(dev) if R > 0 else None
+        if R > 0:
+            spec.ray_dir = self._ray_dir.data_ptr()
         for k, t in self._snap.items():
             setattr(spec, k, t.data_ptr())
         self._spec = spec

@@ -2,15 +2,17 @@
 """
 bench_env.py -- throughput of the closed-loop environment (VecScenarioEnv) and where its step goes.
 
-    python tools/bench_env.py [--out FILE]      # one JSON line per workload on stdout (and appended to FILE)
+    python tools/bench_env.py [--out FILE] [--lidar R]   # one JSON line per workload on stdout (and appended to FILE)
 
 Workloads:
   vehicles  12 500 scenarios x 64 VehicleController entities (synthetic.vehicles_config, 625 distinct
             scenarios each 20 times: building 800 000 host-side entities one by one would dominate the run),
             every vehicle a PolicyAgent: the lean vehicle kernel, one tick per launch.
   xosc      4096 replicas of the reference's 23 test scenarios with the ego a PolicyAgent: the general kernel.
-Observation: K = 8 neighbours within 50 m, lookahead 1 / 2 / 3 s.  The policy is a trivial torch function of
-the observation (steer toward the first lookahead point).
+Observation: K = 8 neighbours within 50 m, lookahead 1 / 2 / 3 s, and with --lidar R > 0 a lidar of R rays
+reaching 50 m (ObsSpec.lidar_rays; 0, the default, leaves the workloads as they were).  The policy is a trivial
+torch function of the observation (steer toward the first lookahead point).  SG_B200_LIB selects the library
+(e.g. a variant built by tools/build_variant.sh); `library` in the record names it.
 
 Reported per workload:
   env_steps_per_s / agent_steps_per_s   step() + policy, host clock over >= 1 s ending in a synchronise
@@ -19,6 +21,7 @@ Reported per workload:
                                         tick (action scatter + one-tick rollout), reward, observe, reset, observe_reset
   fused_us_per_tick                     rollout() of the same scene, 64 ticks in one launch, actions drawn in the kernel
   observe_bytes / observe_GBps          bytes sg_env_observe writes (obs, agent mask, snapshot) over its kernel time
+  lidar_rays / lidar_bytes              R and the bytes of the lidar block (part of observe_bytes)
   device / power_limit_w                the card and its power limit
 """
 from __future__ import annotations
@@ -169,6 +172,8 @@ def measure(name, env):
         "device_us_per_step_total": round(sum(acc.values()), 2),
         "fused_us_per_tick": fused_tick_us,
         "observe_bytes": obs_bytes, "observe_GBps": obs_bytes / (acc["observe"] * 1e-6) / 1e9,
+        "lidar_rays": int(env.obs_spec.lidar_rays), "lidar_bytes": env.N * env.A * 4 * int(env.obs_spec.lidar_rays),
+        "library": os.path.basename(abi.PRODUCT_LIB),
         "device": dev, "power_limit_w": power,
     }
 
@@ -177,10 +182,11 @@ def main():
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     ap.add_argument("--out", default=None, help="also append the JSON lines to this file")
     ap.add_argument("--workloads", default="vehicles,xosc")
+    ap.add_argument("--lidar", type=int, default=0, help="lidar rays R of the observation (0: no lidar block)")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("bench_env.py measures the GPU engine: no CUDA device")
-    obs = ObsSpec(k_neighbours=8, radius=50.0, lookahead=(1.0, 2.0, 3.0))
+    obs = ObsSpec(k_neighbours=8, radius=50.0, lookahead=(1.0, 2.0, 3.0), lidar_rays=args.lidar, lidar_range=50.0)
     for w in args.workloads.split(","):
         t0 = time.time()
         env = {"vehicles": vehicles_env, "xosc": xosc_env}[w](obs)
