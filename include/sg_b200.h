@@ -45,7 +45,7 @@
 extern "C" {
 #endif
 
-#define SG_ABI_VERSION 14
+#define SG_ABI_VERSION 15
 
 /* entity slot kinds (who produces the slot's next pose each tick) */
 enum SgKind {
@@ -393,10 +393,33 @@ int sg_env_observe(const SgScene* scene, const SgParams* params, const SgState* 
    condition of params->terminal holds at this tick, truncated [N] = otherwise (max_length); both are 0
    for the other scenarios.  The conditions are recomputed from the state as the tick decided them:
    collision = n_pair_ticks grew since the snapshot, ego_collision = collided[first_slot],
-   ego_off_road = first_slot absent or not strictly inside the driveable surface. */
+   ego_off_road = first_slot absent or not strictly inside the driveable surface.
+   After several ticks (a branch forked with sg_fork_state and rolled out H ticks) the same evaluation, done
+   once, scores the horizon against the state at the fork: progress = dist_H - dist_0, collision = collided
+   rose at some tick of the horizon (it is sticky), off_road / tracking at the end state (frozen once the
+   scenario is done), rss = flags gained over the horizon, terminated / truncated = how a scenario that
+   finished within the horizon finished.  That is not the sum of the per-tick rewards; with H = 1 it is the
+   reward of one environment step. */
 int sg_env_reward(const SgScene* scene, const SgParams* params, const SgState* state, const SgEnvSpec* spec,
                   float* reward, float* terms, uint8_t* terminated, uint8_t* truncated, int device,
                   void* stream);
+
+/* Fork: copy the state of every scenario of `src` into each of the n_dst states dst[0..n_dst), which must be
+   allocated for the same scene (same N, M: the states do not carry their sizes, so this cannot be checked here)
+   and must not overlap `src` or each other.  Copied: every per-slot plane and per-scenario field of SgState
+   (pose, vel, dist, present, t, prev_t, tick, done, speed, goal_idx, force, cur_own, cur_union, ego_avg_speed,
+   ego_avg_t, ego_max_speed, ego_dist, ego_hits, collided, first_coll_tick, first_coll_pair, n_pair_ticks,
+   rss_state, rss_last, safe_dist, safe_ratio, rss_flags, pid_err; coll_mask for each destination where both
+   sides have one, i.e. non-NULL).  Every destination's event_count is set to 0; events are not copied.  Every
+   destination's trace_cap must be 0 (traces are not copied); the source's trace is ignored.
+   src_spec / dst_spec (both NULL or both given, same n_agents): the snapshot arrays of SgEnvSpec (snap_dist,
+   snap_collided, snap_pair_ticks, snap_rss) are copied the same way, so sg_env_reward of a destination compares
+   against the source's snapshot.  A scenario window (SgScene.plane_stride) applies to the source and every
+   destination alike.  One launch per 64 destinations: each element of the source is read once per launch and
+   stored to every destination.  A rollout of a destination then continues exactly as the source would have:
+   the state is all the tick kernels read. */
+int sg_fork_state(const SgScene* scene, const SgState* src, SgState* const* dst, int n_dst,
+                  const SgEnvSpec* src_spec, SgEnvSpec* const* dst_spec, int device, void* stream);
 
 /* n_ticks x ScenarioGym.step() fused on device (scenario_gym.py:227-254): agents /
    batch replay -> State.step -> RSSDistances -> terminal check -> metrics.  Scenarios

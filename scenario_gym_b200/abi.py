@@ -11,7 +11,7 @@ import math
 import os
 from typing import Dict, Optional
 
-ABI_VERSION = 14
+ABI_VERSION = 15
 
 # SgKind
 KIND_EMPTY, KIND_REPLAY, KIND_AGENT_REPLAY, KIND_VEHICLE, KIND_PEDESTRIAN, KIND_HOST, KIND_PID = range(7)
@@ -337,7 +337,7 @@ def default_params() -> SgParams:
 EXPORTS = [
     "abi_version", "sizeof", "last_error", "default_params", "reset", "rollout",
     "test_box_pairs", "future_collisions", "fill_random_actions", "rollout_host", "host_h2d_bytes",
-    "host_d2h_bytes", "reset_scenarios", "env_observe", "env_reward",
+    "host_d2h_bytes", "reset_scenarios", "env_observe", "env_reward", "fork_state",
 ]
 
 
@@ -372,6 +372,10 @@ def bind(lib: C.CDLL, prefix: str) -> Dict[str, object]:
     get("env_reward", C.c_int,
         [C.POINTER(SgScene), C.POINTER(SgParams), C.POINTER(SgState), C.POINTER(SgEnvSpec), _p, _p, _p, _p,
          C.c_int, _p], required=False)
+    # sg_fork_state: the product exports it; the CPU oracle has no counterpart (a host fork is a numpy copy)
+    get("fork_state", C.c_int,
+        [C.POINTER(SgScene), C.POINTER(SgState), C.POINTER(C.POINTER(SgState)), C.c_int, C.POINTER(SgEnvSpec),
+         C.POINTER(C.POINTER(SgEnvSpec)), C.c_int, _p], required=False)
     get("rollout", C.c_int,
         [C.POINTER(SgScene), C.POINTER(SgParams), C.POINTER(SgState), C.POINTER(SgInputs),
          C.c_int, C.c_int, _p])

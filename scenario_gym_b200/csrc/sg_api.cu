@@ -256,6 +256,49 @@ int sg_env_reward(const SgScene* scene, const SgParams* params, const SgState* s
   return 0;
 }
 
+int sg_fork_state(const SgScene* scene, const SgState* src, SgState* const* dst, int n_dst,
+                  const SgEnvSpec* src_spec, SgEnvSpec* const* dst_spec, int device, void* stream) {
+  if (!scene || !src || !dst) return set_msg("null argument");
+  if (scene->n_slots < 1 || scene->n_slots > 1024) return set_msg("n_slots must be in 1..1024");
+  if (scene->n_scenarios < 1) return set_msg("n_scenarios must be >= 1");
+  if (n_dst < 1) return set_msg("sg_fork_state: n_dst must be >= 1");
+  if (!src_spec != !dst_spec) return set_msg("sg_fork_state: src_spec and dst_spec must both be given or both NULL");
+  SgScene view = *scene;
+  if (view.plane_stride <= 0) {
+    view.plane_stride = (int64_t)scene->n_scenarios * scene->n_slots;
+    view.scenario_base = 0;
+  } else if (view.plane_stride < (int64_t)scene->n_scenarios * scene->n_slots || view.scenario_base < 0) {
+    return set_msg("scenario window: plane_stride smaller than the window / negative scenario_base");
+  }
+  for (int d = -1; d < n_dst; ++d) {
+    const SgState* s = d < 0 ? src : dst[d];
+    if (!s) return set_msg("sg_fork_state: null destination state");
+    if (d >= 0 && s->trace_cap != 0) return set_msg("sg_fork_state: a destination has a trace (trace_cap must be 0)");
+    if (d >= 0 && s == src) return set_msg("sg_fork_state: a destination is the source");
+    if (!s->pose || !s->vel || !s->dist || !s->present || !s->t || !s->prev_t || !s->tick || !s->done || !s->speed ||
+        !s->goal_idx || !s->force || !s->cur_own || !s->cur_union || !s->ego_avg_speed || !s->ego_avg_t ||
+        !s->ego_max_speed || !s->ego_dist || !s->ego_hits || !s->collided || !s->first_coll_tick ||
+        !s->first_coll_pair || !s->n_pair_ticks || !s->event_count || !s->rss_state || !s->rss_last ||
+        !s->safe_dist || !s->safe_ratio || !s->rss_flags || !s->pid_err)
+      return set_msg("sg_fork_state: a state array is missing");
+  }
+  if (src_spec) {
+    for (int d = -1; d < n_dst; ++d) {
+      const SgEnvSpec* e = d < 0 ? src_spec : dst_spec[d];
+      if (!e) return set_msg("sg_fork_state: null destination spec");
+      if (e->n_agents != src_spec->n_agents || e->n_agents < 1 || e->n_agents > scene->n_slots)
+        return set_msg("sg_fork_state: SgEnvSpec.n_agents must be in 1..n_slots and equal on both sides");
+      if (!e->snap_dist || !e->snap_collided || !e->snap_pair_ticks || !e->snap_rss)
+        return set_msg("sg_fork_state: SgEnvSpec snapshot buffers missing");
+    }
+  }
+  cudaError_t err = cudaSetDevice(device);
+  if (err != cudaSuccess) return set_err("cudaSetDevice", err);
+  err = sgi_launch_fork((cudaStream_t)stream, view, *src, dst, n_dst, src_spec, dst_spec);
+  if (err != cudaSuccess) return set_err("sg_fork_kernel launch", err);
+  return 0;
+}
+
 int sg_fill_random_actions(const SgActionRng* rng, int tick0, int n_ticks, int64_t nm, double* out,
                            int device, void* stream) {
   if (!rng || (!out && n_ticks > 0 && nm > 0)) return set_msg("null argument");

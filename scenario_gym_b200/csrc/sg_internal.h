@@ -51,5 +51,8 @@ cudaError_t sgi_launch_env_observe(cudaStream_t s, const SgScene& sc, const SgSt
 cudaError_t sgi_launch_env_reward(cudaStream_t s, const SgScene& sc, const SgParams& p, const SgState& st,
                                   const SgEnvSpec& e, float* reward, float* terms, uint8_t* terminated,
                                   uint8_t* truncated);
+// sg_fork_state (sg_fork.cu); `sc` has its plane stride stated, the arguments are checked
+cudaError_t sgi_launch_fork(cudaStream_t s, const SgScene& sc, const SgState& src, SgState* const* dst, int n_dst,
+                            const SgEnvSpec* src_spec, SgEnvSpec* const* dst_spec);
 cudaError_t sgi_launch_traj(cudaStream_t s, const double* rows, int K, const double* t, int64_t n, int mode,
                             double* pos, uint8_t* ok, double* vel);

@@ -10,7 +10,7 @@ without the built library raises.
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, Optional, Union
+from typing import Dict, Optional, Sequence, Union
 
 import numpy as np
 import torch
@@ -78,8 +78,30 @@ class Engine:
             self._sc.union_x = t.data_ptr()
             self.build_union_on_device()
 
-        # --- state
+        self._alloc_state(coll_matrix)
+
+    @classmethod
+    def sharing_scene(cls, other: "Engine", event_cap: int = 1024, trace_cap: int = 0) -> "Engine":
+        """
+        A second state over ``other``'s device scene: the same scene tensors (nothing is uploaded or packed
+        again), a copy of its parameters and a state of its own, sized like ``other``'s (pair matrix included
+        when ``other`` has one).  What a fork (``fork_into``) needs: branches that do not keep many collision
+        events take a small ``event_cap``.
+        """
+        eng = cls.__new__(cls)
+        eng.lib, eng.device, eng.dev_index = other.lib, other.device, other.dev_index
+        eng.scene = other.scene
+        eng.params = abi.SgParams.from_buffer_copy(other.params)
+        eng.N, eng.M, eng.W = other.N, other.M, other.W
+        eng.event_cap, eng.trace_cap = int(event_cap), int(trace_cap)
+        eng._scene_t = other._scene_t
+        eng._sc = abi.SgScene.from_buffer_copy(other._sc)
+        eng._alloc_state(other._coll_matrix)
+        return eng
+
+    def _alloc_state(self, coll_matrix: bool) -> None:
         N, M, W = self.N, self.M, self.W
+        self._coll_matrix = bool(coll_matrix)
         dims = {"N": N, "M": M, "NM": N * M, "W": W, "E": max(self.event_cap, 1),
                 "T": max(self.trace_cap, 1)}
         self._state_t: Dict[str, torch.Tensor] = {}
@@ -124,6 +146,48 @@ class Engine:
         m = self._scenario_mask(mask)
         self._check(self.lib["reset_scenarios"](C.byref(self._sc), C.byref(self.params), C.byref(self._st),
                                                 m.data_ptr(), self.dev_index, self._stream()))
+
+    def fork_into(self, engines: Sequence["Engine"], spec: Optional[abi.SgEnvSpec] = None,
+                  specs: Optional[Sequence[abi.SgEnvSpec]] = None) -> None:
+        """
+        sg_fork_state: copy this engine's state into every engine of ``engines`` (same scene size, no trace)
+        in one device pass, on the current stream.  The destinations' event counts are set to 0.  With
+        ``spec`` / ``specs`` (the source's SgEnvSpec and one per destination) the snapshot arrays are
+        copied too, so the destinations' env_reward compares against this engine's last observation.
+        """
+        self._check(self.lib["fork_state"](*self.fork_args(engines, spec, specs), self.dev_index, self._stream()))
+
+    def fork_args(self, engines: Sequence["Engine"], spec: Optional[abi.SgEnvSpec] = None,
+                  specs: Optional[Sequence[abi.SgEnvSpec]] = None) -> tuple:
+        """The checked arguments of ``fork_into`` but the device and the stream (callers that fork repeatedly
+        build them once)."""
+        engines = list(engines)
+        if not engines:
+            raise ValueError("fork_into needs at least one destination engine")
+        for e in engines:
+            if not isinstance(e, Engine) or (e.N, e.M) != (self.N, self.M) or e.device != self.device:
+                raise ValueError(f"fork_into: every destination must be an Engine of {self.N} x {self.M} "
+                                 f"slots on {self.device}")
+            if e is self:
+                raise ValueError("fork_into: the source cannot be a destination")
+        if (spec is None) != (specs is None) or (specs is not None and len(specs) != len(engines)):
+            raise ValueError("fork_into: give spec and one spec per destination, or neither")
+        # (ctypes pointers and arrays keep the structures they point to alive)
+        dst = (C.POINTER(abi.SgState) * len(engines))(*[C.pointer(e._fork_view()) for e in engines])
+        src_spec = dst_spec = None
+        if spec is not None:
+            dst_spec = (C.POINTER(abi.SgEnvSpec) * len(specs))(*[C.pointer(s) for s in specs])
+            src_spec = C.pointer(spec)
+        return (C.byref(self._sc), C.byref(self._fork_view()), dst, len(engines), src_spec, dst_spec)
+
+    def _fork_view(self) -> abi.SgState:
+        """The SgState sg_fork_state sees: coll_mask NULL when the pair matrix is not allocated."""
+        if self._coll_matrix:
+            return self._st
+        if getattr(self, "_fork_st", None) is None:
+            self._fork_st = abi.SgState.from_buffer_copy(self._st)
+            self._fork_st.coll_mask = None
+        return self._fork_st
 
     def _scenario_mask(self, mask: torch.Tensor) -> torch.Tensor:
         if not isinstance(mask, torch.Tensor) or mask.device != self.device or mask.numel() != self.N \

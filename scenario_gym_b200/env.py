@@ -177,6 +177,13 @@ class VecScenarioEnv:
         ents = self._gym._entity_of[n]
         return [ents[s] for s in self._gym._env_slots[n]]
 
+    def branches(self, B: int, H: int, final_obs: bool = False) -> "BranchRollout":
+        """
+        A ``BranchRollout`` of ``B`` branches over ``H`` ticks from this env's current state (see there).
+        Everything it needs is allocated here, once.
+        """
+        return BranchRollout(self, B, H, final_obs)
+
     def reset(self) -> Tuple[torch.Tensor, Dict[str, torch.Tensor]]:
         """Every scenario back to its start (sg_reset) and observed; episode counters restart at 0."""
         eng = self._engine
@@ -215,3 +222,139 @@ class VecScenarioEnv:
         eng.tensor("event_count").zero_()  # ego collision events are not kept across steps
         info = dict(self._info, final_obs=self._final_obs, final=self._final, terms=self._terms)
         return self._obs, self._reward, self._terminated.view(torch.bool), self._truncated.view(torch.bool), info
+
+
+def branch_scatter_index(slots: np.ndarray, M: int, B: int, H: int) -> np.ndarray:
+    """
+    Where ``index_copy_`` puts each element of a contiguous ``actions [N, B, H, A, 2]`` in the flat branch action
+    table ``[B][H][2][N*M]`` (plus one trailing element): element (n, b, h, a, c) goes to
+    ``((b*H + h)*2 + c)*N*M + n*M + slots[n, a]``, padding agents (slot -1) to the trailing element, which no
+    rollout reads.  The env's ``_src`` / ``_dst`` scatter of one step, extended over B and H.
+    """
+    slots = np.asarray(slots, np.int64)
+    N, A = slots.shape
+    NM = N * M
+    n = np.arange(N).reshape(N, 1, 1, 1, 1)
+    b = np.arange(B).reshape(1, B, 1, 1, 1)
+    h = np.arange(H).reshape(1, 1, H, 1, 1)
+    c = np.arange(2).reshape(1, 1, 1, 1, 2)
+    s = slots.reshape(N, 1, 1, A, 1)
+    idx = ((b * H + h) * 2 + c) * NM + n * M + s
+    idx = np.where(s >= 0, idx, B * H * 2 * NM)
+    return np.array(np.broadcast_to(idx, (N, B, H, A, 2))).reshape(-1)
+
+
+class BranchRollout:
+    """
+    Branched look-ahead rollouts from a ``VecScenarioEnv``'s live state: ``run(actions)`` forks the env's state
+    (and the snapshot its next reward compares against) into ``B`` branch states in one device pass
+    (``sg_fork_state``), rolls branch ``b`` out for ``H`` ticks with the fused rollout, consuming
+    ``actions[:, b]``, and scores every branch against the state at the fork.  This is what sampling-based
+    planners (random shooting, CEM, MPPI) and counterfactual questions ("would any of these manoeuvres have
+    avoided the collision?") need, at the cost of B x H fused ticks instead of B x H env steps.
+
+    Horizon semantics: ``sg_env_reward`` evaluated once, after the H ticks, against the state at the fork:
+      progress   dist_H - dist_0
+      collision  collided rose at any tick of the horizon (it is sticky)
+      off_road / tracking   at the end state (a branch that finished is frozen where it finished)
+      rss        rss_flags gained a bit over the horizon
+      terminated / truncated   how a branch that finished within the horizon finished (both 0 otherwise)
+    This is not the sum of per-tick rewards.  With H = 1 it is exactly what ``env.step`` computes.  Branches
+    stop where their scenario finishes: ``ticks`` says how many ticks each advanced.
+
+    ``run()`` enqueues everything on the current stream, with no host synchronisation and no device allocation
+    (an ``actions`` tensor that is not contiguous is copied first), and does not touch the env's state, snapshot,
+    observations or episode counters.  It returns views into this object's buffers (overwritten by the next
+    ``run()``), in ``[N, B, ...]`` order, permuted views of ``[B, N, ...]`` storage:
+      ``reward`` [N, B, A] fp32, ``terms`` [N, B, A, 5] fp32, ``terminated`` / ``truncated`` [N, B] bool,
+      ``ticks`` [N, B] int32, ``agent_mask`` [N, B, A] uint8 (the agent is present at the end of the branch),
+      ``final_obs`` [N, B, A, F] fp32 (the observation at the end of the branch, with ``final_obs=True``).
+    """
+
+    def __init__(self, env: VecScenarioEnv, B: int, H: int, final_obs: bool = False):
+        if int(B) != B or int(H) != H or B < 1 or H < 1:
+            raise ValueError(f"branches need B >= 1 and H >= 1, got B={B}, H={H}")
+        B, H = int(B), int(H)
+        src = env._engine
+        # every env state can be forked: the env keeps no trace and sg_fork_state copies everything else
+        assert src.trace_cap == 0, "VecScenarioEnv states have no trace"
+        self.env, self.B, self.H, self.final_obs = env, B, H, bool(final_obs)
+        N, A, M, F = env.N, env.A, src.M, env.n_features
+        dev = env.device
+        self._engines = [type(src).sharing_scene(src, event_cap=1024) for _ in range(B)]
+        # flat action tables [B][H][2][N*M] + one element the padding agents are scattered into
+        size = B * H * 2 * N * M
+        self._flat = {dt: torch.zeros(size + 1, dtype=dt, device=dev) for dt in (torch.float32, torch.float64)}
+        self._tables = {dt: [t[b * H * 2 * N * M:(b + 1) * H * 2 * N * M].view(H, 2, N * M) for b in range(B)]
+                        for dt, t in self._flat.items()}
+        self._index = torch.from_numpy(branch_scatter_index(env._slots_host, M, B, H)).to(dev)
+        # the branches' SgEnvSpecs: the env's, with snapshot arrays of their own
+        self._snaps, self._specs = [], []
+        for _ in range(B):
+            snap = {k: torch.zeros_like(t) for k, t in env._snap.items()}
+            spec = abi.SgEnvSpec.from_buffer_copy(env._spec)
+            for k, t in snap.items():
+                setattr(spec, k, t.data_ptr())
+            self._snaps.append(snap)
+            self._specs.append(spec)
+        self._fork_args = src.fork_args(self._engines, env._spec, self._specs)
+
+        def zeros(*shape, dtype=torch.float32):
+            return torch.zeros(shape, dtype=dtype, device=dev)
+
+        self._reward, self._terms = zeros(B, N, A), zeros(B, N, A, len(abi.ENV_TERMS))
+        self._terminated, self._truncated = zeros(B, N, dtype=torch.uint8), zeros(B, N, dtype=torch.uint8)
+        self._ticks = zeros(B, N, dtype=torch.int32)
+        self._agent_mask = zeros(B, N, A, dtype=torch.uint8)
+        self._final_obs = zeros(B, N, A, F) if self.final_obs else None
+        slots = env._slots_host
+        self._present_idx = torch.from_numpy(
+            (np.arange(N)[:, None] * M + np.maximum(slots, 0)).reshape(-1).astype(np.int64)).to(dev)
+        self._valid = torch.from_numpy((slots >= 0).reshape(-1).astype(np.uint8)).to(dev)
+        out = {"reward": self._reward.permute(1, 0, 2), "terms": self._terms.permute(1, 0, 2, 3),
+               "terminated": self._terminated.view(torch.bool).t(), "truncated": self._truncated.view(torch.bool).t(),
+               "ticks": self._ticks.t(), "agent_mask": self._agent_mask.permute(1, 0, 2)}
+        if self.final_obs:
+            out["final_obs"] = self._final_obs.permute(1, 0, 2, 3)
+        self._out = out
+
+    @property
+    def engines(self):
+        """The B branch engines (their state is the end state of the last ``run()``)."""
+        return list(self._engines)
+
+    def run(self, actions: torch.Tensor) -> Dict[str, torch.Tensor]:
+        """
+        Fork, roll every branch ``H`` ticks and score it; ``actions`` [N, B, H, A, 2] (accel, steer; fp32 or
+        fp64, on the env's device): branch ``b`` consumes ``actions[:, b, h]`` at its h-th tick.  Returns the
+        views described in the class docstring.
+        """
+        env = self.env
+        shape = (env.N, self.B, self.H, env.A, 2)
+        if not isinstance(actions, torch.Tensor):
+            raise ValueError(f"actions must be a torch.Tensor {list(shape)}")
+        if tuple(actions.shape) != shape:
+            raise ValueError(f"actions must have shape {shape}, got {tuple(actions.shape)}")
+        if actions.dtype not in self._flat:
+            raise ValueError(f"actions must be float32 or float64, got {actions.dtype}")
+        if actions.device != env.device:
+            raise ValueError(f"actions must be on {env.device}, got {actions.device}")
+        src = env._engine
+        self._check(src.lib["fork_state"](*self._fork_args, src.dev_index, src._stream()))
+        self._flat[actions.dtype].index_copy_(0, self._index, actions.reshape(-1))
+        tables = self._tables[actions.dtype]
+        tick0 = src.tensor("tick")
+        for b, eng in enumerate(self._engines):
+            eng.rollout(self.H, actions=tables[b])
+            eng.env_reward(self._specs[b], self._reward[b], self._terms[b], self._terminated[b], self._truncated[b])
+            torch.sub(eng.tensor("tick"), tick0, out=self._ticks[b])
+            if self.final_obs:
+                eng.env_observe(self._specs[b], self._final_obs[b], self._agent_mask[b])
+            else:
+                mask = self._agent_mask[b].view(-1)
+                torch.index_select(eng.tensor("present"), 0, self._present_idx, out=mask)
+                mask.mul_(self._valid)
+        return dict(self._out)
+
+    def _check(self, rc: int):
+        self.env._engine._check(rc)
