@@ -45,7 +45,7 @@
 extern "C" {
 #endif
 
-#define SG_ABI_VERSION 15
+#define SG_ABI_VERSION 16
 
 /* entity slot kinds (who produces the slot's next pose each tick) */
 enum SgKind {
@@ -420,6 +420,34 @@ int sg_env_reward(const SgScene* scene, const SgParams* params, const SgState* s
    the state is all the tick kernels read. */
 int sg_fork_state(const SgScene* scene, const SgState* src, SgState* const* dst, int n_dst,
                   const SgEnvSpec* src_spec, SgEnvSpec* const* dst_spec, int device, void* stream);
+
+/* MPPI planning over the branch action tables (model-predictive path integral: sample perturbed action sequences,
+   weight each by exp(reward / lambda), move the mean to the weighted average).  With A = spec->n_agents, agent a
+   of scenario n is slot s = spec->agent_slot[n*A + a] (s = -1: padding, never read or written here).  The mean
+   mu [N][H][A][2] is fp64, component c = 0 accel, 1 steer.  `table` is the flat branch action table
+   [B][H][2][N*M] that sg_rollout consumes per branch (table_b = table + b*H*2*N*M): fp32, or fp64 with
+   table_is_f64 != 0.  All arrays are device memory but `sigma` (host, [2]).
+
+   sg_plan_sample: for every real agent, branch b and tick h, with i = ((n*A + a)*B + b)*H + h (int64) and
+   (z0, z1) = the engine's counter-based N(0, 1) pair of (seed, i, k) (splitmix64 + Box-Muller, the SocialForce
+   noise of SgParams.sf_std_*), eps_c = sigma_c * z_c for b >= 1 and 0 for b = 0 (branch 0 is the mean):
+     table_b[h][c][n*M + s] = mu[n][h][a][c] + eps_c, rounded once to the table's type.
+   No other table entry is written and nothing is clipped (the VehicleController clips actions).  Scenarios with
+   reset[n] != 0 (reset NULL: none) have their mean zeroed first.  sigma finite and >= 0, k >= 0.
+
+   sg_plan_update: reward [B][N][A] fp32 (sg_env_reward of each branch after its H ticks).  In fp64, summing in
+   ascending b: Rmax = max_b R_b, w_b = exp((R_b - Rmax) / lambda), eps_hat_b = (double)table_b[h][c][n*M + s]
+   - mu_in[n][h][a][c] (the noise is read back from the table, not stored), mu' = mu_in + (sum_b w_b eps_hat_b) /
+   (sum_b w_b).  best_branch [N][A] int32 = the smallest b with R_b = Rmax, best_reward [N][A] = Rmax.
+   finish = 0: mu_out = mu'.  finish != 0 (the last iteration of a planning step): action [N][A][2] fp32 =
+   mu'[n][0][a], and mu_out holds the mean of the next step, shifted one tick: mu_out[h] = mu'[h + 1],
+   mu_out[H-1] = 0.  mu_in and mu_out must not overlap; lambda finite and > 0. */
+int sg_plan_sample(const SgEnvSpec* spec, int n_scenarios, int n_slots, int n_branches, int horizon, uint64_t seed,
+                   int k, const double* sigma, double* mu, const uint8_t* reset, void* table, int table_is_f64,
+                   int device, void* stream);
+int sg_plan_update(const SgEnvSpec* spec, int n_scenarios, int n_slots, int n_branches, int horizon, double lambda,
+                   const float* reward, const void* table, int table_is_f64, const double* mu_in, double* mu_out,
+                   int finish, float* action, int32_t* best_branch, float* best_reward, int device, void* stream);
 
 /* n_ticks x ScenarioGym.step() fused on device (scenario_gym.py:227-254): agents /
    batch replay -> State.step -> RSSDistances -> terminal check -> metrics.  Scenarios

@@ -8,7 +8,7 @@ gym / engine does (there is no CPU fallback).
 """
 from .actions import FixedTAction, ScenarioAction, UpdateStateVariableAction, UserDefinedAction
 from .entity import BoundingBox, CatalogEntry, Entity, MiscObject, Pedestrian, Vehicle
-from .env import BranchRollout, ObsSpec, VecScenarioEnv
+from .env import BranchRollout, MPPIPlanner, ObsSpec, VecScenarioEnv
 from .gym import ScenarioGym
 from .plugins import (RSS, Action, ActionTableAgent, Agent, CollisionMetric, CollisionObservation,
                       CombinedSensor, Controller, GlobalCollisionDetector, combine_observations,

@@ -11,7 +11,7 @@ import math
 import os
 from typing import Dict, Optional
 
-ABI_VERSION = 15
+ABI_VERSION = 16
 
 # SgKind
 KIND_EMPTY, KIND_REPLAY, KIND_AGENT_REPLAY, KIND_VEHICLE, KIND_PEDESTRIAN, KIND_HOST, KIND_PID = range(7)
@@ -337,7 +337,7 @@ def default_params() -> SgParams:
 EXPORTS = [
     "abi_version", "sizeof", "last_error", "default_params", "reset", "rollout",
     "test_box_pairs", "future_collisions", "fill_random_actions", "rollout_host", "host_h2d_bytes",
-    "host_d2h_bytes", "reset_scenarios", "env_observe", "env_reward", "fork_state",
+    "host_d2h_bytes", "reset_scenarios", "env_observe", "env_reward", "fork_state", "plan_sample", "plan_update",
 ]
 
 
@@ -376,6 +376,13 @@ def bind(lib: C.CDLL, prefix: str) -> Dict[str, object]:
     get("fork_state", C.c_int,
         [C.POINTER(SgScene), C.POINTER(SgState), C.POINTER(C.POINTER(SgState)), C.c_int, C.POINTER(SgEnvSpec),
          C.POINTER(C.POINTER(SgEnvSpec)), C.c_int, _p], required=False)
+    # sg_plan_sample / sg_plan_update: the product exports them; the CPU oracle has none (tests restate them)
+    get("plan_sample", C.c_int,
+        [C.POINTER(SgEnvSpec), C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint64, C.c_int, C.POINTER(C.c_double), _p,
+         _p, _p, C.c_int, C.c_int, _p], required=False)
+    get("plan_update", C.c_int,
+        [C.POINTER(SgEnvSpec), C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, _p, _p, C.c_int, _p, _p, C.c_int,
+         _p, _p, _p, C.c_int, _p], required=False)
     get("rollout", C.c_int,
         [C.POINTER(SgScene), C.POINTER(SgParams), C.POINTER(SgState), C.POINTER(SgInputs),
          C.c_int, C.c_int, _p])

@@ -299,6 +299,56 @@ int sg_fork_state(const SgScene* scene, const SgState* src, SgState* const* dst,
   return 0;
 }
 
+// the checks sg_plan_sample and sg_plan_update share
+static int check_plan(const char* who, const SgEnvSpec* e, int N, int M, int B, int H, const void* table) {
+  if (!e || !table) return set_msg("null argument");
+  if (M < 1 || M > 1024) return set_msg("n_slots must be in 1..1024");
+  if (N < 1) return set_msg("n_scenarios must be >= 1");
+  if (B < 1 || H < 1) {
+    snprintf(g_err, sizeof(g_err), "%s: n_branches and horizon must be >= 1 (got %d, %d)", who, B, H);
+    return -1;
+  }
+  if (e->n_agents < 1 || e->n_agents > M) return set_msg("SgEnvSpec.n_agents must be in 1..n_slots");
+  if (!e->agent_slot) return set_msg("SgEnvSpec.agent_slot missing");
+  return 0;
+}
+
+int sg_plan_sample(const SgEnvSpec* spec, int n_scenarios, int n_slots, int n_branches, int horizon, uint64_t seed,
+                   int k, const double* sigma, double* mu, const uint8_t* reset, void* table, int table_is_f64,
+                   int device, void* stream) {
+  int rc = check_plan("sg_plan_sample", spec, n_scenarios, n_slots, n_branches, horizon, table);
+  if (rc) return rc;
+  if (!sigma || !mu) return set_msg("null argument");
+  if (k < 0) return set_msg("sg_plan_sample: k must be >= 0");
+  for (int c = 0; c < 2; ++c)
+    if (!isfinite(sigma[c]) || sigma[c] < 0.0) return set_msg("sg_plan_sample: sigma must be finite and >= 0");
+  cudaError_t err = cudaSetDevice(device);
+  if (err != cudaSuccess) return set_err("cudaSetDevice", err);
+  err = sgi_launch_plan_sample((cudaStream_t)stream, *spec, n_scenarios, n_slots, n_branches, horizon, seed, k, sigma,
+                               mu, reset, table, table_is_f64 != 0);
+  if (err != cudaSuccess) return set_err("sg_plan_sample_kernel launch", err);
+  return 0;
+}
+
+int sg_plan_update(const SgEnvSpec* spec, int n_scenarios, int n_slots, int n_branches, int horizon, double lambda,
+                   const float* reward, const void* table, int table_is_f64, const double* mu_in, double* mu_out,
+                   int finish, float* action, int32_t* best_branch, float* best_reward, int device, void* stream) {
+  int rc = check_plan("sg_plan_update", spec, n_scenarios, n_slots, n_branches, horizon, table);
+  if (rc) return rc;
+  if (!reward || !mu_in || !mu_out || !best_branch || !best_reward || (finish && !action))
+    return set_msg("null argument");
+  if (!isfinite(lambda) || !(lambda > 0.0)) return set_msg("sg_plan_update: lambda must be finite and > 0");
+  const size_t mu_bytes = (size_t)n_scenarios * horizon * spec->n_agents * 2 * sizeof(double);
+  const char *i0 = (const char*)mu_in, *o0 = (const char*)mu_out;
+  if (i0 < o0 + mu_bytes && o0 < i0 + mu_bytes) return set_msg("sg_plan_update: mu_in and mu_out overlap");
+  cudaError_t err = cudaSetDevice(device);
+  if (err != cudaSuccess) return set_err("cudaSetDevice", err);
+  err = sgi_launch_plan_update((cudaStream_t)stream, *spec, n_scenarios, n_slots, n_branches, horizon, lambda, reward,
+                               table, table_is_f64 != 0, mu_in, mu_out, finish != 0, action, best_branch, best_reward);
+  if (err != cudaSuccess) return set_err("sg_plan_update_kernel launch", err);
+  return 0;
+}
+
 int sg_fill_random_actions(const SgActionRng* rng, int tick0, int n_ticks, int64_t nm, double* out,
                            int device, void* stream) {
   if (!rng || (!out && n_ticks > 0 && nm > 0)) return set_msg("null argument");

@@ -54,5 +54,13 @@ cudaError_t sgi_launch_env_reward(cudaStream_t s, const SgScene& sc, const SgPar
 // sg_fork_state (sg_fork.cu); `sc` has its plane stride stated, the arguments are checked
 cudaError_t sgi_launch_fork(cudaStream_t s, const SgScene& sc, const SgState& src, SgState* const* dst, int n_dst,
                             const SgEnvSpec* src_spec, SgEnvSpec* const* dst_spec);
+// sg_plan_sample / sg_plan_update (sg_plan.cu); the arguments are checked
+cudaError_t sgi_launch_plan_sample(cudaStream_t s, const SgEnvSpec& e, int N, int M, int B, int H, uint64_t seed,
+                                   int k, const double sigma[2], double* mu, const uint8_t* reset, void* table,
+                                   bool table_f64);
+cudaError_t sgi_launch_plan_update(cudaStream_t s, const SgEnvSpec& e, int N, int M, int B, int H, double lambda,
+                                   const float* reward, const void* table, bool table_f64, const double* mu_in,
+                                   double* mu_out, bool finish, float* action, int32_t* best_branch,
+                                   float* best_reward);
 cudaError_t sgi_launch_traj(cudaStream_t s, const double* rows, int K, const double* t, int64_t n, int mode,
                             double* pos, uint8_t* ok, double* vel);

@@ -211,6 +211,28 @@ class Engine:
                                            terminated.data_ptr(), truncated.data_ptr(), self.dev_index,
                                            self._stream()))
 
+    def plan_sample(self, spec: abi.SgEnvSpec, B: int, H: int, seed: int, k: int, sigma, mu: torch.Tensor,
+                    reset: Optional[torch.Tensor], table: torch.Tensor) -> None:
+        """sg_plan_sample: the B branches' actions drawn around the mean ``mu`` (fp64 [N, H, A, 2]) into the flat
+        branch table ``table`` ([B][H][2][N*M], fp32 or fp64); ``reset`` (uint8 / bool [N] or None): the scenarios
+        whose mean is zeroed first."""
+        sig = (C.c_double * 2)(float(sigma[0]), float(sigma[1]))
+        r = None if reset is None else self._scenario_mask(reset).data_ptr()
+        self._check(self.lib["plan_sample"](C.byref(spec), self.N, self.M, int(B), int(H), int(seed) & (2**64 - 1),
+                                            int(k), sig, mu.data_ptr(), r, table.data_ptr(),
+                                            int(table.dtype == torch.float64), self.dev_index, self._stream()))
+
+    def plan_update(self, spec: abi.SgEnvSpec, B: int, H: int, lam: float, reward: torch.Tensor,
+                    table: torch.Tensor, mu_in: torch.Tensor, mu_out: torch.Tensor, finish: bool,
+                    action: Optional[torch.Tensor], best_branch: torch.Tensor, best_reward: torch.Tensor) -> None:
+        """sg_plan_update: the mean ``mu_in`` moved to the reward-weighted average of the branches (``reward`` fp32
+        [B, N, A]) into ``mu_out``; with ``finish`` also the first action (fp32 [N, A, 2]) and the shift."""
+        self._check(self.lib["plan_update"](C.byref(spec), self.N, self.M, int(B), int(H), float(lam),
+                                            reward.data_ptr(), table.data_ptr(), int(table.dtype == torch.float64),
+                                            mu_in.data_ptr(), mu_out.data_ptr(), int(bool(finish)),
+                                            None if action is None else action.data_ptr(), best_branch.data_ptr(),
+                                            best_reward.data_ptr(), self.dev_index, self._stream()))
+
     def build_union_on_device(self) -> torch.Tensor:
         """
         Recompute the resident BatchReplayEntity union table from the uploaded control points and knot

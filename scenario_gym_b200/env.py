@@ -148,6 +148,7 @@ class VecScenarioEnv:
         self._terminated, self._truncated = zeros(N, dtype=torch.uint8), zeros(N, dtype=torch.uint8)
         self._finished = zeros(N, dtype=torch.uint8)
         self._episode = zeros(N, dtype=torch.int64)
+        self._resets = 0  # reset() calls so far
         self._final = {k: torch.zeros_like(eng.tensor(f)) for k, f in _FINAL_FIELDS.items()}
         self._snap = {"snap_dist": zeros(N * self.A, dtype=torch.float64),
                       "snap_collided": zeros(N * self.A, dtype=torch.uint8),
@@ -184,11 +185,18 @@ class VecScenarioEnv:
         """
         return BranchRollout(self, B, H, final_obs)
 
+    def planner(self, B: int = 64, H: int = 30, sigma: Sequence[float] = (1.0, 0.1), temperature: float = 1.0,
+                iterations: int = 1, seed: int = 0) -> "MPPIPlanner":
+        """An ``MPPIPlanner`` over ``B`` branches of ``H`` ticks from this env (see there).  Everything it needs is
+        allocated here, once."""
+        return MPPIPlanner(self, B, H, sigma, temperature, iterations, seed)
+
     def reset(self) -> Tuple[torch.Tensor, Dict[str, torch.Tensor]]:
         """Every scenario back to its start (sg_reset) and observed; episode counters restart at 0."""
         eng = self._engine
         eng.reset()
         self._episode.zero_()
+        self._resets += 1  # (a planner cannot see this reset in the episode counters when they were 0)
         eng.env_observe(self._spec, self._obs, self._agent_mask)
         return self._obs, dict(self._info)
 
@@ -339,10 +347,14 @@ class BranchRollout:
             raise ValueError(f"actions must be float32 or float64, got {actions.dtype}")
         if actions.device != env.device:
             raise ValueError(f"actions must be on {env.device}, got {actions.device}")
-        src = env._engine
-        self._check(src.lib["fork_state"](*self._fork_args, src.dev_index, src._stream()))
         self._flat[actions.dtype].index_copy_(0, self._index, actions.reshape(-1))
-        tables = self._tables[actions.dtype]
+        self._roll(self._tables[actions.dtype])
+        return dict(self._out)
+
+    def _roll(self, tables: List[torch.Tensor]) -> None:
+        """Fork, roll branch ``b`` ``H`` ticks on ``tables[b]`` ([H][2][N*M]) and score it into the buffers."""
+        src = self.env._engine
+        self._check(src.lib["fork_state"](*self._fork_args, src.dev_index, src._stream()))
         tick0 = src.tensor("tick")
         for b, eng in enumerate(self._engines):
             eng.rollout(self.H, actions=tables[b])
@@ -354,7 +366,89 @@ class BranchRollout:
                 mask = self._agent_mask[b].view(-1)
                 torch.index_select(eng.tensor("present"), 0, self._present_idx, out=mask)
                 mask.mul_(self._valid)
-        return dict(self._out)
 
     def _check(self, rc: int):
         self.env._engine._check(rc)
+
+
+class MPPIPlanner:
+    """
+    MPPI (model-predictive path integral) planning on the device, over a ``BranchRollout`` of ``B`` branches and
+    ``H`` ticks: ``plan()`` repeats ``iterations`` times
+      sample   ``sg_plan_sample`` draws branch b's actions, mean + sigma * N(0, 1) (branch 0: the mean itself),
+               straight into the branch action table (no [N, B, H, A, 2] tensor, no scatter);
+      roll     fork the env's state, roll every branch H ticks and score it (``BranchRollout``'s horizon reward);
+      update   ``sg_plan_update`` moves the mean to the average of the branches weighted by
+               exp((R_b - max R) / temperature), reading the noise back from the same table (it is never stored),
+    per agent and independently.  The last update also returns the first action of the refined mean and shifts the
+    mean one tick for the next ``plan()`` (its last tick starts at 0).  The mean of a scenario whose episode
+    changed since the last ``plan()`` (auto-reset in ``env.step``, or ``env.reset()``) restarts at 0.  Semantics:
+    include/sg_b200.h, sg_plan_sample / sg_plan_update.
+
+    The noise is a pure function of (seed, agent, branch, tick, call counter), so two planners with the same seed
+    driving equal envs plan the same actions.  ``plan()`` enqueues everything on the current stream, with no host
+    synchronisation and no allocation, and leaves the env's state, snapshot, observations and episode counters
+    alone.  Each agent plans for its own reward (there is no scenario-level objective), and actions are bounded
+    only by the controller's clipping.
+    """
+
+    def __init__(self, env: VecScenarioEnv, B: int = 64, H: int = 30, sigma: Sequence[float] = (1.0, 0.1),
+                 temperature: float = 1.0, iterations: int = 1, seed: int = 0):
+        if int(B) != B or B < 2:
+            raise ValueError(f"the planner needs B >= 2 branches (branch 0 is the mean), got B={B}")
+        if int(H) != H or H < 1:
+            raise ValueError(f"the planner needs H >= 1, got H={H}")
+        if int(iterations) != iterations or iterations < 1:
+            raise ValueError(f"iterations must be >= 1, got {iterations}")
+        sigma = tuple(float(s) for s in sigma)
+        if len(sigma) != 2 or not all(math.isfinite(s) and s >= 0.0 for s in sigma):
+            raise ValueError(f"sigma must be two finite values >= 0 (accel, steer), got {sigma}")
+        temperature = float(temperature)
+        if not (math.isfinite(temperature) and temperature > 0.0):
+            raise ValueError(f"temperature must be finite and > 0, got {temperature}")
+        self.env, self.B, self.H = env, int(B), int(H)
+        self.sigma, self.temperature, self.iterations, self.seed = sigma, temperature, int(iterations), int(seed)
+        self.branches = BranchRollout(env, self.B, self.H)
+        br, N, A, dev = self.branches, env.N, env.A, env.device
+        # the table type the branch rollouts consume without a conversion
+        dt = torch.float64 if br._engines[0]._wants_f64_table() else torch.float32
+        self._table, self._tables = br._flat[dt], br._tables[dt]
+        self._mean = torch.zeros(2, N, self.H, A, 2, dtype=torch.float64, device=dev)  # ping-pong
+        self._cur = 0
+        self._action = torch.zeros(N, A, 2, device=dev)
+        self._best_branch = torch.zeros(N, A, dtype=torch.int32, device=dev)
+        self._best_reward = torch.zeros(N, A, device=dev)
+        self._seen = env._episode.clone()
+        self._resets = env._resets
+        self._changed = torch.zeros(N, dtype=torch.bool, device=dev)
+        self._all = torch.ones(N, dtype=torch.uint8, device=dev)
+        self._k = 0  # sample passes so far: the noise counter
+
+    def plan(self) -> Tuple[torch.Tensor, Dict[str, torch.Tensor]]:
+        """
+        One planning step from the env's current state.  Returns views into the planner's buffers (overwritten by
+        the next ``plan()``): ``actions`` [N, A, 2] fp32, the first action of the refined mean, and ``info`` with
+        ``mean`` [N, H, A, 2] fp64 (the refined mean shifted one tick: where the next ``plan()`` starts),
+        ``reward`` [N, B, A] (the branch rewards of the last iteration), ``best_branch`` [N, A] int32 and
+        ``best_reward`` [N, A] fp32 (the smallest b with the largest reward, and that reward).
+        """
+        env, br, B, H = self.env, self.branches, self.B, self.H
+        eng, spec = env._engine, env._spec
+        if self._resets != env._resets:
+            self._resets = env._resets
+            reset = self._all
+        else:
+            reset = torch.ne(env._episode, self._seen, out=self._changed)
+        self._seen.copy_(env._episode)
+        for it in range(self.iterations):
+            mu = self._mean[self._cur]
+            eng.plan_sample(spec, B, H, self.seed, self._k, self.sigma, mu, reset if it == 0 else None, self._table)
+            self._k += 1
+            br._roll(self._tables)
+            self._cur ^= 1
+            last = it == self.iterations - 1
+            eng.plan_update(spec, B, H, self.temperature, br._reward, self._table, mu, self._mean[self._cur], last,
+                            self._action if last else None, self._best_branch, self._best_reward)
+        info = {"mean": self._mean[self._cur], "reward": br._out["reward"], "best_branch": self._best_branch,
+                "best_reward": self._best_reward}
+        return self._action, info
