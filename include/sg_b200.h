@@ -45,7 +45,7 @@
 extern "C" {
 #endif
 
-#define SG_ABI_VERSION 16
+#define SG_ABI_VERSION 17
 
 /* entity slot kinds (who produces the slot's next pose each tick) */
 enum SgKind {
@@ -338,8 +338,35 @@ typedef struct SgInputs {
                 So a touching corner or a ray along an edge hits, an origin inside another box reads 0 and
                 boxes without width / size act as segments / points.  Reading = min(ray_range, smallest hit
                 distance over j) in fp64, rounded once to fp32 (ray_range when nothing is hit).
-   The row is F = 4 + 3*L + 10*K + (road ? 2 : 0) + R floats; with R = 0 it is the row without the lidar
-   block, bit for bit.  Absent / padding agents get zero rows.  Reward terms (after a tick, against the snapshot the last
+     map        (map_edges = Km > 0) the Km nearest road-network edges, 10 floats each, between the road block
+                and the lidar block.  Map table: built once per network r (= rn_of[n]) from the scene's soups,
+                walking surface k = 0, 1, 2 (driveable, walkable, impenetrable), then its polygons, then their
+                edges: zero-length edges are dropped, edges with the same endpoints in either direction are kept
+                once (the first occurrence, with its orientation), and every kept edge carries flag bit k for each
+                surface k it occurs in (a building's edges are walkable and impenetrable).  Edges that only
+                partly overlap are not merged.  Edge index e = the edge's position in its network's table.
+                Distance of (x, y) to edge (x0, y0) -> (x1, y1), this operation order, no FMA:
+                  dx = x1 - x0, dy = y1 - y0, wx = x - x0, wy = y - y0, L2 = dx*dx + dy*dy,
+                  t = L2 > 0 ? (wx*dx + wy*dy) / L2 : 0, clamped to [0, 1], qx = x0 + t*dx, qy = y0 + t*dy,
+                  d2 = (qx - x)*(qx - x) + (qy - y)*(qy - y).
+                Selected: the Km smallest (d2, e) with d2 < map_radius^2, ascending (ties: the lower e).  The
+                selection depends on x and y only, so every implementation selects the same edges.  Per edge:
+                rot(qx - x, qy - y), rot(x0 - x, y0 - y), rot(x1 - x, y1 - y), the 3 surface flags as 0 / 1, 1.
+                Missing entries, and every entry of a scenario without a network, are zeros.
+                Culling grid (an implementation aid that must not change the selection): network r covers
+                nx x ny square cells of side `cell` from (ox, oy); the cell of a coordinate v along an axis is
+                ix(v) = floor((v - ox) / cell) clamped to [0, nx - 1] (fp64, the builder and the device compute
+                it alike).  An edge is listed in every cell of [ix(bx0 - m), ix(bx1 + m)] x [iy(by0 - m),
+                iy(by1 + m)], (bx0, by0) - (bx1, by1) its bounding box and m the grid's margin, and map_cell0
+                holds the lower corner of that range.  A query from (x, y) visits [ix(x - w), ix(x + w)] x
+                [iy(y - w), iy(y + w)], w = map_radius + m, and tests an edge only in the first visited cell
+                that lists it: (max(ix(x - w), cell0.x), max(iy(y - w), cell0.y)).  The exact d2 test decides.
+                Rounding moves the computed nearest point off the edge's bounding box by a few ulps of the
+                coordinates; any m above that (the builder takes 1e-9 x (1 + largest |coordinate| + radius))
+                makes the visited cells cover every edge with d2 < map_radius^2, because ix() is monotone and
+                clamping keeps overlapping ranges overlapping.
+   The row is F = 4 + 3*L + 10*K + (road ? 2 : 0) + 10*Km + R floats; with Km = 0 and R = 0 it is the row
+   without the map and lidar blocks, bit for bit.  Absent / padding agents get zero rows.  Reward terms (after a tick, against the snapshot the last
    observe took): progress = dist - dist_snap; collision = collided rose 0 -> 1; off_road = network has
    driveable area and the present slot is not strictly inside it; tracking = -|(x, y) - position_at_t(own
    trajectory, t, clamped)[:2]|; rss = the slot is the ego and rss_flags gained a bit.  Absent / padding
@@ -363,6 +390,19 @@ typedef struct SgEnvSpec {
   int32_t _pad0;
   double ray_range;          /* metres, finite and > 0 when R > 0 */
   const double* ray_dir;     /* [R][2] device: unit directions in the agent frame (see above) */
+  /* map block (between the road and lidar blocks; read by sg_env_observe only).  All pointers device memory,
+     needed when Km > 0 and the scene has networks; the table of network r is rows map_off[r] .. map_off[r+1] */
+  int32_t map_edges;             /* Km, 0..32 (0: no map block) */
+  int32_t map_networks;          /* networks the table was built for: must be SgScene.n_networks */
+  double map_radius;             /* metres, finite and > 0 when Km > 0 */
+  const int64_t* map_off;        /* [map_networks + 1] */
+  const double* map_seg;         /* [rows][4] x0, y0, x1, y1 */
+  const uint8_t* map_flags;      /* [rows] bit k: the edge occurs in surface k */
+  const int32_t* map_cell0;      /* [rows][2] lower corner (ix, iy) of the cells listing the edge */
+  const double* map_grid;        /* [map_networks][4] ox, oy, cell (> 0), margin m (>= 0) */
+  const int64_t* map_dims;       /* [map_networks][3] nx, ny (>= 1), first cell in map_cell_off */
+  const int64_t* map_cell_off;   /* [total cells + 1] CSR: cell c lists map_cell_edge[map_cell_off[c] ..) */
+  const int32_t* map_cell_edge;  /* edge indices e within the network, ascending per cell */
 } SgEnvSpec;
 
 int sg_abi_version(void);

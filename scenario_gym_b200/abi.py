@@ -11,7 +11,7 @@ import math
 import os
 from typing import Dict, Optional
 
-ABI_VERSION = 16
+ABI_VERSION = 17
 
 # SgKind
 KIND_EMPTY, KIND_REPLAY, KIND_AGENT_REPLAY, KIND_VEHICLE, KIND_PEDESTRIAN, KIND_HOST, KIND_PID = range(7)
@@ -233,6 +233,17 @@ class SgEnvSpec(C.Structure):
         ("_pad0", C.c_int32),
         ("ray_range", C.c_double),
         ("ray_dir", _p),
+        ("map_edges", C.c_int32),
+        ("map_networks", C.c_int32),
+        ("map_radius", C.c_double),
+        ("map_off", _p),
+        ("map_seg", _p),
+        ("map_flags", _p),
+        ("map_cell0", _p),
+        ("map_grid", _p),
+        ("map_dims", _p),
+        ("map_cell_off", _p),
+        ("map_cell_edge", _p),
     ]
 
 
@@ -240,9 +251,114 @@ class SgEnvSpec(C.Structure):
 ENV_TERMS = ("progress", "collision", "off_road", "tracking", "rss")
 
 
-def env_n_features(k_neighbours: int, n_lookahead: int, road: bool, n_rays: int = 0) -> int:
+def env_n_features(k_neighbours: int, n_lookahead: int, road: bool, n_rays: int = 0, map_edges: int = 0) -> int:
     """Floats per observation row of sg_env_observe (include/sg_b200.h, SgEnvSpec)."""
-    return 4 + 3 * n_lookahead + 10 * k_neighbours + (2 if road else 0) + n_rays
+    return 4 + 3 * n_lookahead + 10 * k_neighbours + (2 if road else 0) + 10 * map_edges + n_rays
+
+
+# the arrays of the map block's table and grid, in SgEnvSpec order (the field names of SgEnvSpec)
+MAP_FIELDS = ("map_off", "map_seg", "map_flags", "map_cell0", "map_grid", "map_dims", "map_cell_off", "map_cell_edge")
+# most grid cells one network may have (a finer cell size is widened to stay below it)
+MAP_MAX_CELLS = 1 << 20
+
+
+def map_network_edges(rn_poly_off, rn_edge_off, rn_edges, r: int):
+    """The map table of network r (include/sg_b200.h, SgEnvSpec, map block): (seg [E, 4] fp64, flags [E] uint8),
+    the edges of its three surfaces walked surface, polygon, edge; zero-length edges dropped; edges with the same
+    endpoints (either direction) kept once, at their first occurrence and with its orientation, flag bit k set
+    for every surface k they occur in."""
+    import numpy as np
+
+    segs, surf = [], []
+    for k in range(3):
+        p0, p1 = int(rn_poly_off[3 * r + k]), int(rn_poly_off[3 * r + k + 1])
+        e0, e1 = int(rn_edge_off[p0]), int(rn_edge_off[p1])
+        segs.append(np.asarray(rn_edges[e0:e1], np.float64).reshape(-1, 4))
+        surf.append(np.full(e1 - e0, k, np.int64))
+    seg, surf = np.concatenate(segs), np.concatenate(surf)
+    keep = ~((seg[:, 0] == seg[:, 2]) & (seg[:, 1] == seg[:, 3]))
+    seg, surf = seg[keep], surf[keep]
+    if len(seg) == 0:
+        return np.zeros((0, 4)), np.zeros(0, np.uint8)
+    # same endpoints in either direction: compare the endpoints in lexicographic order (-0.0 counts as 0.0)
+    key = seg + 0.0
+    swap = (key[:, 0] > key[:, 2]) | ((key[:, 0] == key[:, 2]) & (key[:, 1] > key[:, 3]))
+    key[swap] = key[swap][:, [2, 3, 0, 1]]
+    key = np.ascontiguousarray(key).view(np.dtype((np.void, 32))).reshape(-1)
+    _, first, inv = np.unique(key, return_index=True, return_inverse=True)
+    flags = np.zeros(len(first), np.uint8)
+    np.bitwise_or.at(flags, inv.reshape(-1), (1 << surf).astype(np.uint8))
+    order = np.argsort(first, kind="stable")
+    return np.ascontiguousarray(seg[first[order]]), flags[order]
+
+
+def map_cell_index(v, o: float, cell: float, n: int):
+    """The grid cell of coordinates v along one axis: floor((v - o) / cell) clamped to [0, n - 1] (int64)."""
+    import numpy as np
+
+    return np.clip(np.floor((np.asarray(v, np.float64) - o) / cell), 0, n - 1).astype(np.int64)
+
+
+def map_table(rn_poly_off, rn_edge_off, rn_edges, radius: float, cell: Optional[float] = None):
+    """
+    The map block's table and culling grid of every network of a scene (SgScene.rn_* as numpy arrays), as the
+    numpy arrays of ``MAP_FIELDS``.  Per network: margin m = 1e-9 * (1 + largest |coordinate| + radius), origin
+    the table's bounding box minus m, square cells of side ``cell`` (None: radius / 2, widened where the network
+    would need more than ``MAP_MAX_CELLS`` cells; ``math.inf``: a single cell, i.e. brute force), every edge
+    listed, in ascending order, in the cells its bounding box widened by m overlaps (include/sg_b200.h).
+    """
+    import numpy as np
+
+    radius = float(radius)
+    if not (math.isfinite(radius) and radius > 0.0):
+        raise ValueError(f"map radius must be finite and > 0, got {radius}")
+    if cell is not None and not float(cell) > 0.0:
+        raise ValueError(f"map grid cell size must be > 0, got {cell}")
+    R = (len(rn_poly_off) - 1) // 3
+    off, segs, flags, cell0, grid, dims, cell_off, cell_edge = [0], [], [], [], [], [], [np.zeros(1, np.int64)], []
+    n_cells = n_listed = 0
+    for r in range(R):
+        seg, fl = map_network_edges(rn_poly_off, rn_edge_off, rn_edges, r)
+        E = len(seg)
+        bx0, bx1 = np.minimum(seg[:, 0], seg[:, 2]), np.maximum(seg[:, 0], seg[:, 2])
+        by0, by1 = np.minimum(seg[:, 1], seg[:, 3]), np.maximum(seg[:, 1], seg[:, 3])
+        big = float(np.abs(seg).max()) if E else 0.0
+        m = 1e-9 * (1.0 + big + radius)
+        ox, oy = (float(bx0.min()) - m, float(by0.min()) - m) if E else (0.0, 0.0)
+        ex, ey = (float(bx1.max()) + m - ox, float(by1.max()) + m - oy) if E else (0.0, 0.0)
+        c = 0.5 * radius if cell is None else float(cell)
+        if math.isfinite(c):
+            c = max(c, math.sqrt(ex * ey / MAP_MAX_CELLS), max(ex, ey) / MAP_MAX_CELLS)
+        nx = int(math.floor(ex / c)) + 1 if E else 1
+        ny = int(math.floor(ey / c)) + 1 if E else 1
+        ix0, ix1 = map_cell_index(bx0 - m, ox, c, nx), map_cell_index(bx1 + m, ox, c, nx)
+        iy0, iy1 = map_cell_index(by0 - m, oy, c, ny), map_cell_index(by1 + m, oy, c, ny)
+        wx, cnt = ix1 - ix0 + 1, (ix1 - ix0 + 1) * (iy1 - iy0 + 1)
+        ed = np.repeat(np.arange(E, dtype=np.int64), cnt)
+        local = np.arange(len(ed), dtype=np.int64) - np.repeat(np.cumsum(cnt) - cnt, cnt)
+        cid = (iy0[ed] + local // wx[ed]) * nx + ix0[ed] + local % wx[ed]
+        order = np.lexsort((ed, cid))
+        counts = np.bincount(cid, minlength=nx * ny)
+        off.append(off[-1] + E)
+        segs.append(seg)
+        flags.append(fl)
+        cell0.append(np.stack([ix0, iy0], 1).astype(np.int32).reshape(-1, 2))
+        grid.append([ox, oy, c, m])
+        dims.append([nx, ny, n_cells])
+        cell_off.append(n_listed + np.cumsum(counts))
+        cell_edge.append(ed[order].astype(np.int32))
+        n_cells += nx * ny
+        n_listed += len(ed)
+    return {
+        "map_off": np.array(off, np.int64),
+        "map_seg": np.ascontiguousarray(np.concatenate(segs) if segs else np.zeros((0, 4)), np.float64),
+        "map_flags": np.concatenate(flags).astype(np.uint8) if flags else np.zeros(0, np.uint8),
+        "map_cell0": np.ascontiguousarray(np.concatenate(cell0) if cell0 else np.zeros((0, 2)), np.int32),
+        "map_grid": np.array(grid, np.float64).reshape(R, 4),
+        "map_dims": np.array(dims, np.int64).reshape(R, 3),
+        "map_cell_off": np.concatenate(cell_off).astype(np.int64),
+        "map_cell_edge": np.concatenate(cell_edge).astype(np.int32) if cell_edge else np.zeros(0, np.int32),
+    }
 
 
 def lidar_directions(n_rays: int):

@@ -222,6 +222,16 @@ static int check_env(const SgScene* sc, const SgParams* p, const SgState* st, co
       return set_msg("SgEnvSpec.ray_range must be finite and > 0 when n_rays > 0");
     if (!e->ray_dir) return set_msg("SgEnvSpec.ray_dir missing (n_rays > 0)");
   }
+  if (e->map_edges < 0 || e->map_edges > 32) return set_msg("SgEnvSpec.map_edges must be in 0..32");
+  if (e->map_edges > 0) {
+    if (!isfinite(e->map_radius) || !(e->map_radius > 0.0))
+      return set_msg("SgEnvSpec.map_radius must be finite and > 0 when map_edges > 0");
+    if (e->map_networks != sc->n_networks)
+      return set_msg("SgEnvSpec.map_networks differs from the scene's n_networks (the map table is per network)");
+    if (sc->n_networks > 0 && (!e->map_off || !e->map_seg || !e->map_flags || !e->map_cell0 || !e->map_grid ||
+                               !e->map_dims || !e->map_cell_off || !e->map_cell_edge))
+      return set_msg("SgEnvSpec: map table / grid pointers missing (map_edges > 0)");
+  }
   *view = *sc;
   view->plane_stride = (int64_t)sc->n_scenarios * sc->n_slots;
   view->scenario_base = 0;

@@ -365,6 +365,125 @@ static cudaError_t launch_lidar(cudaStream_t s, const SgScene& sc, const SgState
   return cudaGetLastError();
 }
 
+// ---- map block of sg_env_observe (semantics and grid conditions in include/sg_b200.h, SgEnvSpec) ----
+#define SG_MAP_THREADS 128
+
+// the grid cell of coordinate v along one axis: floor((v - o) / cell) clamped to [0, n - 1] (the builder's rule)
+static __device__ __forceinline__ int map_cell(double v, double o, double cell, int64_t n) {
+  const double f = floor((v - o) / cell);
+  return (int)(f < 0.0 ? 0.0 : (f > (double)(n - 1) ? (double)(n - 1) : f));
+}
+
+// sg_env_map_kernel: one thread per (scenario, agent).  A present agent of a scenario with a network visits the
+// cells its square [x +- w] x [y +- w] overlaps, tests each listed edge in the first visited cell that lists it
+// (so an edge spanning several cells is inserted once), keeps the KCAP smallest (d2, e) in a register-resident
+// sorted list (the observe kernel's unrolled insertion) and writes the 10 * Km map columns [col, col + 10 Km) of
+// its row, zeros for missing entries.  Absent and padding agents are skipped: the observe kernel zero-filled
+// their rows.  A table built with a single cell makes this the brute-force search over every edge of the network.
+template <int KCAP>
+__global__ void __launch_bounds__(SG_MAP_THREADS)
+sg_env_map_kernel(SgScene sc, SgState st, SgEnvSpec e, const uint8_t* __restrict__ mask, float* __restrict__ obs,
+                  int F, int col) {
+  const int64_t ia = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  const int A = e.n_agents, M = sc.n_slots, Km = e.map_edges;
+  if (ia >= (int64_t)sc.n_scenarios * A) return;
+  const int n = (int)(ia / A);
+  if (mask && !mask[n]) return;
+  const int slot = e.agent_slot[ia];
+  if (slot < 0 || slot >= M) return;
+  const int64_t nm = sc.plane_stride, i = (int64_t)n * M + slot;
+  if (!st.present[i]) return;
+  const double x = st.pose[i], y = st.pose[nm + i];
+  const int r = sc.rn_of ? sc.rn_of[n] : -1;
+  double bd[KCAP];
+  int bs[KCAP];
+#pragma unroll
+  for (int q = 0; q < KCAP; ++q) { bd[q] = INFINITY; bs[q] = INT_MAX; }
+  int64_t row0 = 0;
+  if (r >= 0) {
+    row0 = e.map_off[r];
+    const double r2 = e.map_radius * e.map_radius;
+    const double ox = e.map_grid[4 * r], oy = e.map_grid[4 * r + 1], cell = e.map_grid[4 * r + 2];
+    const double w = e.map_radius + e.map_grid[4 * r + 3];
+    const int64_t nx = e.map_dims[3 * r], ny = e.map_dims[3 * r + 1], c0 = e.map_dims[3 * r + 2];
+    const int ix0 = map_cell(x - w, ox, cell, nx), ix1 = map_cell(x + w, ox, cell, nx);
+    const int iy0 = map_cell(y - w, oy, cell, ny), iy1 = map_cell(y + w, oy, cell, ny);
+    for (int cy = iy0; cy <= iy1; ++cy) {
+      for (int cx = ix0; cx <= ix1; ++cx) {
+        const int64_t c = c0 + cy * nx + cx;
+        const int64_t k1 = e.map_cell_off[c + 1];
+        for (int64_t k = e.map_cell_off[c]; k < k1; ++k) {
+          const int ed = e.map_cell_edge[k];
+          const int2 lo = reinterpret_cast<const int2*>(e.map_cell0)[row0 + ed];
+          if ((lo.x > ix0 ? lo.x : ix0) != cx || (lo.y > iy0 ? lo.y : iy0) != cy) continue;  // tested elsewhere
+          const double2 p0 = reinterpret_cast<const double2*>(e.map_seg)[2 * (row0 + ed)];
+          const double2 p1 = reinterpret_cast<const double2*>(e.map_seg)[2 * (row0 + ed) + 1];
+          const double dx = p1.x - p0.x, dy = p1.y - p0.y, wx = x - p0.x, wy = y - p0.y;
+          const double L2 = dx * dx + dy * dy;
+          double t = L2 > 0.0 ? (wx * dx + wy * dy) / L2 : 0.0;
+          t = t < 0.0 ? 0.0 : (t > 1.0 ? 1.0 : t);
+          const double qx = p0.x + t * dx, qy = p0.y + t * dy;
+          const double d2 = (qx - x) * (qx - x) + (qy - y) * (qy - y);
+          if (!(d2 < r2)) continue;
+          if (!(d2 < bd[KCAP - 1] || (d2 == bd[KCAP - 1] && ed < bs[KCAP - 1]))) continue;
+          double cd = d2;
+          int cj = ed;
+#pragma unroll
+          for (int q = 0; q < KCAP; ++q) {
+            const bool lt = cd < bd[q] || (cd == bd[q] && cj < bs[q]);
+            const double td = bd[q];
+            const int tj = bs[q];
+            bd[q] = lt ? cd : td; bs[q] = lt ? cj : tj;
+            cd = lt ? td : cd; cj = lt ? tj : cj;
+          }
+        }
+      }
+    }
+  }
+  double s = 0.0, c = 1.0;
+  sincos(st.pose[3 * nm + i], &s, &c);
+  float* out = obs + ia * F + col;
+#pragma unroll
+  for (int q = 0; q < KCAP; ++q) {
+    if (q >= Km) break;
+    float* m = out + 10 * q;
+    const int ed = bs[q];
+    if (ed == INT_MAX) {
+#pragma unroll
+      for (int k = 0; k < 10; ++k) m[k] = 0.0f;
+      continue;
+    }
+    const double2 p0 = reinterpret_cast<const double2*>(e.map_seg)[2 * (row0 + ed)];
+    const double2 p1 = reinterpret_cast<const double2*>(e.map_seg)[2 * (row0 + ed) + 1];
+    const double dx = p1.x - p0.x, dy = p1.y - p0.y, wx = x - p0.x, wy = y - p0.y;
+    const double L2 = dx * dx + dy * dy;
+    double t = L2 > 0.0 ? (wx * dx + wy * dy) / L2 : 0.0;
+    t = t < 0.0 ? 0.0 : (t > 1.0 ? 1.0 : t);
+    const double ux = (p0.x + t * dx) - x, uy = (p0.y + t * dy) - y;
+    const double ax = p0.x - x, ay = p0.y - y, bx = p1.x - x, by = p1.y - y;
+    const unsigned fl = e.map_flags[row0 + ed];
+    m[0] = (float)(c * ux + s * uy);
+    m[1] = (float)(-s * ux + c * uy);
+    m[2] = (float)(c * ax + s * ay);
+    m[3] = (float)(-s * ax + c * ay);
+    m[4] = (float)(c * bx + s * by);
+    m[5] = (float)(-s * bx + c * by);
+    m[6] = (fl & 1u) ? 1.0f : 0.0f;
+    m[7] = (fl & 2u) ? 1.0f : 0.0f;
+    m[8] = (fl & 4u) ? 1.0f : 0.0f;
+    m[9] = 1.0f;
+  }
+}
+
+template <int KCAP>
+static cudaError_t launch_map_t(cudaStream_t s, const SgScene& sc, const SgState& st, const SgEnvSpec& e,
+                                const uint8_t* mask, float* obs, int F, int col) {
+  const int64_t n = (int64_t)sc.n_scenarios * e.n_agents;
+  sg_env_map_kernel<KCAP><<<(unsigned)((n + SG_MAP_THREADS - 1) / SG_MAP_THREADS), SG_MAP_THREADS, 0, s>>>(
+      sc, st, e, mask, obs, F, col);
+  return cudaGetLastError();
+}
+
 template <int KCAP>
 static cudaError_t launch_observe_t(cudaStream_t s, const SgScene& sc, const SgState& st, const SgEnvSpec& e,
                                     const uint8_t* mask, float* obs, uint8_t* agent_mask, int F) {
@@ -377,12 +496,20 @@ static cudaError_t launch_observe_t(cudaStream_t s, const SgScene& sc, const SgS
 
 cudaError_t sgi_launch_env_observe(cudaStream_t s, const SgScene& sc, const SgState& st, const SgEnvSpec& e,
                                    const uint8_t* mask, float* obs, uint8_t* agent_mask) {
-  const int F = 4 + 3 * e.n_lookahead + 10 * e.k_neighbours + (e.road ? 2 : 0) + e.n_rays;
+  const int col = 4 + 3 * e.n_lookahead + 10 * e.k_neighbours + (e.road ? 2 : 0);  // first map column
+  const int F = col + 10 * e.map_edges + e.n_rays;
   cudaError_t err;
   if (e.k_neighbours <= 8) err = launch_observe_t<8>(s, sc, st, e, mask, obs, agent_mask, F);
   else if (e.k_neighbours <= 16) err = launch_observe_t<16>(s, sc, st, e, mask, obs, agent_mask, F);
   else err = launch_observe_t<32>(s, sc, st, e, mask, obs, agent_mask, F);
-  if (err != cudaSuccess || e.n_rays <= 0) return err;
+  if (err != cudaSuccess) return err;
+  if (e.map_edges > 0) {  // (after the zero rows, same stream; the map columns only)
+    if (e.map_edges <= 8) err = launch_map_t<8>(s, sc, st, e, mask, obs, F, col);
+    else if (e.map_edges <= 16) err = launch_map_t<16>(s, sc, st, e, mask, obs, F, col);
+    else err = launch_map_t<32>(s, sc, st, e, mask, obs, F, col);
+    if (err != cudaSuccess) return err;
+  }
+  if (e.n_rays <= 0) return err;
   return launch_lidar(s, sc, st, e, mask, obs, F);  // (after the row prefix and the zero rows, same stream)
 }
 

@@ -36,18 +36,23 @@ class ObsSpec:
     entities within ``radius`` metres (<= 0: no cut-off), its own trajectory ``lookahead`` seconds ahead
     (at most 8 times), with ``road`` whether it is on the driveable surface and how far its edge is, and with
     ``lidar_rays`` = R (0..256) a planar lidar: R rays at angles 2 pi k / R from its heading, each reading the
-    distance to the first box of another present entity, at most ``lidar_range`` metres."""
+    distance to the first box of another present entity, at most ``lidar_range`` metres.  With ``map_edges`` = Km
+    (0..32) it also sees the Km road-network edges (of the driveable, walkable and impenetrable surfaces) nearest to
+    it within ``map_radius`` metres: the nearest point and both end points in its frame, which surfaces the edge
+    bounds, and a valid flag (10 floats each, between the road block and the lidar)."""
     k_neighbours: int = 8
     radius: float = 50.0
     lookahead: Sequence[float] = (1.0, 2.0, 3.0)
     road: bool = False
     lidar_rays: int = 0
     lidar_range: float = 50.0
+    map_edges: int = 0
+    map_radius: float = 50.0
 
     @property
     def n_features(self) -> int:
         return abi.env_n_features(int(self.k_neighbours), len(self.lookahead), bool(self.road),
-                                  int(self.lidar_rays))
+                                  int(self.lidar_rays), int(self.map_edges))
 
 
 def _ego_policy(scenario: Scenario, entity: Entity):
@@ -95,6 +100,11 @@ class VecScenarioEnv:
             raise ValueError(f"ObsSpec: lidar_rays must be in 0..256, got {self.obs_spec.lidar_rays}")
         if R > 0 and not (math.isfinite(float(self.obs_spec.lidar_range)) and float(self.obs_spec.lidar_range) > 0):
             raise ValueError(f"ObsSpec: lidar_range must be finite and > 0, got {self.obs_spec.lidar_range}")
+        Km = int(self.obs_spec.map_edges)
+        if Km != self.obs_spec.map_edges or not 0 <= Km <= 32:
+            raise ValueError(f"ObsSpec: map_edges must be in 0..32, got {self.obs_spec.map_edges}")
+        if Km > 0 and not (math.isfinite(float(self.obs_spec.map_radius)) and float(self.obs_spec.map_radius) > 0):
+            raise ValueError(f"ObsSpec: map_radius must be finite and > 0, got {self.obs_spec.map_radius}")
         w = dict(DEFAULT_REWARD_WEIGHTS)
         if isinstance(reward_weights, Mapping):
             unknown = set(reward_weights) - set(abi.ENV_TERMS)
@@ -167,6 +177,18 @@ class VecScenarioEnv:
         self._ray_dir = torch.from_numpy(abi.lidar_directions(R)).to(dev) if R > 0 else None
         if R > 0:
             spec.ray_dir = self._ray_dir.data_ptr()
+        spec.map_edges, spec.map_radius = Km, float(self.obs_spec.map_radius)
+        # the map table and its grid, built once per network from the lowered scene (the env keeps them alive)
+        self._map = {}
+        if Km > 0:
+            sc = eng.scene
+            spec.map_networks = sc.n_networks
+            if sc.n_networks > 0:
+                table = abi.map_table(sc.rn_poly_off, sc.rn_edge_off, sc.rn_edges, spec.map_radius)
+                for k, a in table.items():  # (an empty array still gets an address)
+                    a = a if a.size else np.zeros((1,) + a.shape[1:], a.dtype)
+                    self._map[k] = torch.from_numpy(np.ascontiguousarray(a)).to(dev)
+                    setattr(spec, k, self._map[k].data_ptr())
         for k, t in self._snap.items():
             setattr(spec, k, t.data_ptr())
         self._spec = spec

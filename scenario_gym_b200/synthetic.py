@@ -228,3 +228,74 @@ def crowd_config(seed: int, N: int, M: int = 1024, T: int = 128, dt: float = 1.0
         name=name, N=N, M=M, T=T, dt=dt, x0=x0, y0=y0, h0=h0, v0=v0, box=box, kind=kind,
         etype=etype, speed_desired=speed_desired, goal=goal,
     )
+
+
+def grid_town(seed: int, half_extent: float = 220.0, center=(0.0, 0.0), spacing: float = 80.0, lanes: int = 2,
+              lane_width: float = 3.5, pavement: float = 3.0, buildings: float = 0.8):
+    """
+    A seeded synthetic town (``RoadNetwork``) covering the square ``center +- half_extent``: a grid of roads
+    ``spacing`` metres apart, rotated by an angle and shifted by an offset drawn from ``seed``.  Every road
+    segment between two intersections is a ``Road`` split into ``2 * lanes`` ``Lane`` strips (which share their
+    edges with each other and with the road); every crossing is an ``Intersection`` square; both sides of a road
+    segment carry a ``Pavement`` strip; every block holds up to four ``Building`` lots (each present with
+    probability ``buildings``) with jittered footprints.  The same seed gives the same network, float for float.
+    """
+    from .road_network import Building, Intersection, Lane, PolygonArea, Pavement, Road, RoadNetwork
+
+    rng = np.random.default_rng(seed)
+    theta = rng.uniform(0.0, 0.5 * np.pi)
+    shift = rng.uniform(-0.5 * spacing, 0.5 * spacing, 2)
+    c, s = np.cos(theta), np.sin(theta)
+    cx0, cy0 = float(center[0]), float(center[1])
+
+    def world(pts):  # local grid coordinates -> world (the same local point always gives the same floats)
+        return [(cx0 + c * (u + shift[0]) - s * (v + shift[1]), cy0 + s * (u + shift[0]) + c * (v + shift[1]))
+                for u, v in pts]
+
+    def rect(u0, v0, u1, v1):
+        return PolygonArea(world([(u0, v0), (u1, v0), (u1, v1), (u0, v1)]))
+
+    hw = lanes * lane_width  # half width of a road
+    n = int(np.ceil((half_extent * np.sqrt(2.0) + spacing) / spacing))
+    lines = [k * spacing for k in range(-n, n + 1)]
+    roads, inters, paves, blds = [], [], [], []
+    for i, a in enumerate(lines):
+        for j, b in enumerate(lines):
+            inters.append(Intersection(f"x{i}_{j}", rect(a - hw, b - hw, a + hw, b + hw)))
+            if i + 1 < len(lines):  # along u from this crossing to the next, and along v (transposed)
+                a1 = lines[i + 1]
+                for axis in (0, 1):
+                    def box(p0, q0, p1, q1):
+                        return rect(p0, q0, p1, q1) if axis == 0 else rect(q0, p0, q1, p1)
+                    u0, u1 = a + hw, a1 - hw
+                    lane_list = [Lane(f"l{axis}_{i}_{j}_{k}", box(u0, b - hw + k * lane_width, u1,
+                                                                  b - hw + (k + 1) * lane_width))
+                                 for k in range(2 * lanes)]
+                    roads.append(Road(f"r{axis}_{i}_{j}", box(u0, b - hw, u1, b + hw), lanes=lane_list))
+                    paves.append(Pavement(f"p{axis}_{i}_{j}_0", box(u0, b - hw - pavement, u1, b - hw)))
+                    paves.append(Pavement(f"p{axis}_{i}_{j}_1", box(u0, b + hw, u1, b + hw + pavement)))
+            if i + 1 < len(lines) and j + 1 < len(lines):  # the block between four roads: 2 x 2 lots
+                u0, v0 = a + hw + pavement, b + hw + pavement
+                side = 0.5 * (spacing - 2.0 * (hw + pavement))
+                for lu in range(2):
+                    for lv in range(2):
+                        keep = rng.random() < buildings
+                        inset = rng.uniform(1.0, 4.0, 4)
+                        jitter = rng.uniform(-1.0, 1.0, (4, 2))
+                        if not keep:
+                            continue
+                        p0, q0 = u0 + lu * side, v0 + lv * side
+                        corners = [(p0 + inset[0], q0 + inset[1]), (p0 + side - inset[2], q0 + inset[1]),
+                                   (p0 + side - inset[2], q0 + side - inset[3]), (p0 + inset[0], q0 + side - inset[3])]
+                        pts = [(u + du, v + dv) for (u, v), (du, dv) in zip(corners, jitter)]
+                        blds.append(Building(f"b{i}_{j}_{lu}{lv}", PolygonArea(world(pts))))
+    # keep the geometries that reach into the covered square (with a road's width of slack)
+    lim = half_extent + spacing
+
+    def near(g):
+        ext = g.boundary.exterior
+        return (np.abs(ext[:, 0] - cx0) <= lim).any() and (np.abs(ext[:, 1] - cy0) <= lim).any()
+
+    keep_roads = [r for r in roads if near(r)]
+    return RoadNetwork(name=f"grid_town_{seed}", roads=keep_roads, intersections=[g for g in inters if near(g)],
+                       pavements=[g for g in paves if near(g)], buildings=[g for g in blds if near(g)])

@@ -2,7 +2,8 @@
 """
 bench_env.py -- throughput of the closed-loop environment (VecScenarioEnv) and where its step goes.
 
-    python tools/bench_env.py [--out FILE] [--lidar R]   # one JSON line per workload on stdout (and appended to FILE)
+    python tools/bench_env.py [--out FILE] [--lidar R] [--map Km]   # one JSON line per workload on stdout (and
+                                                                     # appended to FILE)
 
 Workloads:
   vehicles  12 500 scenarios x 64 VehicleController entities (synthetic.vehicles_config, 625 distinct
@@ -10,7 +11,10 @@ Workloads:
             every vehicle a PolicyAgent: the lean vehicle kernel, one tick per launch.
   xosc      4096 replicas of the reference's 23 test scenarios with the ego a PolicyAgent: the general kernel.
 Observation: K = 8 neighbours within 50 m, lookahead 1 / 2 / 3 s, and with --lidar R > 0 a lidar of R rays
-reaching 50 m (ObsSpec.lidar_rays; 0, the default, leaves the workloads as they were).  The policy is a trivial
+reaching 50 m (ObsSpec.lidar_rays; 0, the default, leaves the workloads as they were).  With --map Km > 0 every
+scenario drives over a synthetic town (synthetic.grid_town: the vehicles' 400 m square, or one town over the 23 test
+scenes' trajectory points, 0.5 .. 99.5 % range) and observes its Km nearest road-network edges within 50 m (ObsSpec.map_edges; 0, the default, attaches no
+town and leaves the workloads as they were).  The policy is a trivial
 torch function of the observation (steer toward the first lookahead point).  SG_B200_LIB selects the library
 (e.g. a variant built by tools/build_variant.sh); `library` in the record names it.
 
@@ -22,12 +26,17 @@ Reported per workload:
   fused_us_per_tick                     rollout() of the same scene, 64 ticks in one launch, actions drawn in the kernel
   observe_bytes / observe_GBps          bytes sg_env_observe writes (obs, agent mask, snapshot) over its kernel time
   lidar_rays / lidar_bytes              R and the bytes of the lidar block (part of observe_bytes)
+  map_edges / map_table_edges / map_bytes   Km, the edges of the town's map table, the bytes of the map block
+  map_us / map_brute_us                 the map kernel's time per observe (observe with the map block minus observe
+                                        without it, CUDA events over 50 calls each), with the env's culling grid and
+                                        with the same table built as a single cell (brute force, same kernel)
   device / power_limit_w                the card and its power limit
 """
 from __future__ import annotations
 
 import argparse
 import json
+import math
 import os
 import subprocess
 import sys
@@ -38,6 +47,7 @@ REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if REPO not in sys.path:
     sys.path.insert(0, REPO)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 from scenario_gym_b200 import (BoundingBox, CatalogEntry, Entity, ObsSpec, Pedestrian, PolicyAgent,  # noqa: E402
@@ -56,8 +66,9 @@ def vehicles_env(obs):
     cfg = synthetic.vehicles_config(seed=0, N=distinct, M=M, T=256)
     rows = synthetic.two_knot_rows(cfg).reshape(distinct, M, 2, 7)
     ce = CatalogEntry(None, "car1", "car", "Vehicle", BoundingBox(*synthetic.CAR1_BOX))
+    town = synthetic.grid_town(seed=0, half_extent=200.0) if obs.map_edges > 0 else None
     scs = [Scenario([Vehicle(ce, trajectory=Trajectory(rows[n, m]), ref="ego" if m == 0 else f"entity_{m}")
-                     for m in range(M)]) for n in range(distinct)]
+                     for m in range(M)], road_network=town) for n in range(distinct)]
     return VecScenarioEnv(scs * reps, create_agent=lambda s, e: PolicyAgent(e), timestep=cfg.dt, obs=obs)
 
 
@@ -76,6 +87,13 @@ def xosc_env(obs):
             ce = CatalogEntry(None, "entry", None, ctype, BoundingBox(*[float(v) for v in inp["box"][i]]))
             ents.append(C(ce, trajectory=Trajectory(inp[f"traj{i}"]), ref=man[name]["refs"][i]))
         scs.append(Scenario(ents))
+    if obs.map_edges > 0:  # one town over the test scenes: the 0.5 .. 99.5 % range of their trajectory points
+        # (one scene has a stray point thousands of km away, which a town cannot sensibly cover)
+        xy = np.concatenate([np.asarray(e.trajectory.data)[:, 1:3] for sc in scs for e in sc.entities])
+        lo, hi = np.quantile(xy, 0.005, axis=0), np.quantile(xy, 0.995, axis=0)
+        town = synthetic.grid_town(seed=0, half_extent=float((hi - lo).max()) / 2 + 20.0, center=(lo + hi) / 2)
+        for sc in scs:
+            sc.road_network = town
     return VecScenarioEnv([scs[k % len(scs)] for k in range(4096)], obs=obs)
 
 
@@ -160,6 +178,8 @@ def measure(name, env):
     torch.cuda.synchronize()
     fused_tick_us = e0.elapsed_time(e1) * 1e3 / 64
     assert int(fused.get("tick").min()) == 64, "every scenario must run the 64 timed ticks"
+    del fused
+    maps = map_times(env) if env.obs_spec.map_edges > 0 else {}
     F = env.n_features
     obs_bytes = env.N * env.A * (4 * F + 1 + 9) + env.N * 9
     dev, power = card()
@@ -173,9 +193,41 @@ def measure(name, env):
         "fused_us_per_tick": fused_tick_us,
         "observe_bytes": obs_bytes, "observe_GBps": obs_bytes / (acc["observe"] * 1e-6) / 1e9,
         "lidar_rays": int(env.obs_spec.lidar_rays), "lidar_bytes": env.N * env.A * 4 * int(env.obs_spec.lidar_rays),
+        "map_edges": int(env.obs_spec.map_edges), "map_bytes": env.N * env.A * 40 * int(env.obs_spec.map_edges),
+        **maps,
         "library": os.path.basename(abi.PRODUCT_LIB),
         "device": dev, "power_limit_w": power,
     }
+
+
+def map_times(env):
+    """The map kernel's time per observe: observe with the env's spec minus observe with map_edges = 0, and the
+    same with the table built as a single cell (brute force through the same kernel)."""
+    eng, sc, stream = env._engine, env._engine.scene, torch.cuda.current_stream()
+    plain = abi.SgEnvSpec.from_buffer_copy(env._spec)
+    plain.map_edges = 0
+    brute = abi.SgEnvSpec.from_buffer_copy(env._spec)
+    table = abi.map_table(sc.rn_poly_off, sc.rn_edge_off, sc.rn_edges, env.obs_spec.map_radius, cell=math.inf)
+    keep = {k: torch.from_numpy(np.ascontiguousarray(a)).to(env.device) for k, a in table.items()}
+    for k, t in keep.items():
+        setattr(brute, k, t.data_ptr())
+
+    def observe_us(spec, reps=50):
+        for _ in range(3):
+            eng.env_observe(spec, env._obs, env._agent_mask)
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record(stream)
+        for _ in range(reps):
+            eng.env_observe(spec, env._obs, env._agent_mask)
+        e1.record(stream)
+        torch.cuda.synchronize()
+        return e0.elapsed_time(e1) * 1e3 / reps
+
+    base, grid, flat = observe_us(plain), observe_us(env._spec), observe_us(brute)
+    dims = env._map["map_dims"].cpu().numpy()
+    return {"map_table_edges": int(env._map["map_off"][-1].item()), "map_grid_cells": int((dims[:, 0] * dims[:, 1]).sum()),
+            "map_cell_m": float(env._map["map_grid"][0, 2].item()), "observe_no_map_us": round(base, 2),
+            "map_us": round(grid - base, 2), "map_brute_us": round(flat - base, 2)}
 
 
 def main():
@@ -183,10 +235,12 @@ def main():
     ap.add_argument("--out", default=None, help="also append the JSON lines to this file")
     ap.add_argument("--workloads", default="vehicles,xosc")
     ap.add_argument("--lidar", type=int, default=0, help="lidar rays R of the observation (0: no lidar block)")
+    ap.add_argument("--map", type=int, default=0, help="map edges Km of the observation (0: no town, no map block)")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("bench_env.py measures the GPU engine: no CUDA device")
-    obs = ObsSpec(k_neighbours=8, radius=50.0, lookahead=(1.0, 2.0, 3.0), lidar_rays=args.lidar, lidar_range=50.0)
+    obs = ObsSpec(k_neighbours=8, radius=50.0, lookahead=(1.0, 2.0, 3.0), lidar_rays=args.lidar, lidar_range=50.0,
+                  map_edges=args.map, map_radius=50.0)
     for w in args.workloads.split(","):
         t0 = time.time()
         env = {"vehicles": vehicles_env, "xosc": xosc_env}[w](obs)
