@@ -45,7 +45,7 @@
 extern "C" {
 #endif
 
-#define SG_ABI_VERSION 17
+#define SG_ABI_VERSION 18
 
 /* entity slot kinds (who produces the slot's next pose each tick) */
 enum SgKind {
@@ -155,7 +155,9 @@ typedef struct SgScene {
   int64_t n_route_pts; /* total points in route_xy         */
   /* OR of (1u << SgKind) over all slots, or 0 = unspecified (always valid).  A non-zero mask
      lets the library pick a specialised kernel; {VEHICLE[,EMPTY]} additionally promises that
-     every vehicle slot is present at reset (its trajectory covers t0). */
+     every vehicle slot is present at reset (its trajectory covers t0, and, for a reset at a later
+     start time (sg_reset_scenarios_init), that start time: the caller keeps its start windows inside
+     every vehicle's logged span). */
   uint32_t kind_mask;
   uint32_t scene_flags; /* SgSceneFlag bits */
   const uint8_t* kind;   /* [N*M] SgKind */
@@ -407,7 +409,7 @@ typedef struct SgEnvSpec {
 
 int sg_abi_version(void);
 /* sizeof() of the ABI structs so bindings can verify their mirror: which = 0 SgParams,
-   1 SgScene, 2 SgState, 3 SgInputs, 4 SgEvent, 5 SgActionRng, 6 SgHostResults, 7 SgEnvSpec */
+   1 SgScene, 2 SgState, 3 SgInputs, 4 SgEvent, 5 SgActionRng, 6 SgHostResults, 7 SgEnvSpec, 8 SgResetInit */
 int64_t sg_sizeof(int which);
 const char* sg_last_error(void);
 void sg_default_params(SgParams* p);
@@ -420,6 +422,48 @@ int sg_reset(const SgScene* scene, const SgParams* params, SgState* state, int d
    field of every other scenario is left as it was, and event_count is not touched. */
 int sg_reset_scenarios(const SgScene* scene, const SgParams* params, SgState* state, const uint8_t* mask,
                        int device, void* stream);
+
+/* Randomised start of the scenarios a masked reset selects (sg_reset_scenarios_init). */
+typedef struct SgResetInit {
+  const double* t_start;      /* [N] device, absolute start times; NULL: drawn from start_window */
+  const double* start_window; /* [N] device, seconds >= 0; NULL (and no t_start): every start is t0 */
+  const int64_t* counter;     /* [N] device: the draw index k of scenario n (read only; the caller advances it) */
+  const uint8_t* perturb;     /* [N*M] device: non-zero for the slots whose start is perturbed; NULL: none */
+  double sigma[4];            /* std of: along-heading offset (m), across (m), heading (rad), speed (m/s); >= 0 */
+  uint64_t seed;
+} SgResetInit;
+
+/* sg_reset_scenarios at a start time of each selected scenario's own, with the agents' starts optionally
+   perturbed.  Scenario n (mask[n] != 0, mask NULL: all) with global index g = scenario_base + n and draw
+   index k = counter[n]; every noise value is the engine's counter-based stream (splitmix64 + Box-Muller, the
+   SocialForce noise of SgParams.sf_std_*), keyed by (seed, counter c, tick value 2k or 2k + 1 taken mod 2^32).
+   - Start time T: t_start[n] if t_start is given; else t0[n] + u * start_window[n] (fp64, that operation order,
+     no FMA) with u = (a >> 11) * 2^-53 in [0, 1), a = the first splitmix64 value of the stream's key for counter
+     c = -1 - g and tick value 2k (the uniform that precedes Box-Muller; counter -1 - g is never a slot index);
+     else t0[n].
+   - The reset at T is sg_reset of the scene whose t0[n] is T, field for field: presence, poses, velocities,
+     controller speed, prev_t = T - 0.1, cursors, the RSS pass at reset (with its T != 0 rule) and the ego
+     metrics.  (The tick kernels read the time from the state, never t0, so the episode then continues exactly
+     as one of a scene logged from T.)  Pedestrians restart at goal_idx 0 of their route, as at any t0: their
+     routes are not re-targeted to the later start.
+   - Perturbation of slot i = n*M + s with perturb[i] != 0 that is present at T: (z0, z1) = noise of counter
+     (g*M + s) and tick value 2k, (z2, z3) of the same counter and 2k + 1.  With (x, y, h) the reset's pose,
+     (c, s) = (cos h, sin h), v0 = norm2(vx, vy) and the operation order written here, no FMA:
+       position, when sigma[0] or sigma[1] != 0:  lon = sigma[0]*z0, lat = sigma[1]*z1,
+                  x += c*lon - s*lat,  y += s*lon + c*lat;
+       heading, when sigma[2] != 0:  dh = sigma[2]*z2, h' = h + dh;
+       speed, when sigma[2] or sigma[3] != 0:  v = max(0, v0 + sigma[3]*z3); with (cd, sd) = (cos dh, sin dh)
+                  (dh = 0 when sigma[2] = 0), f = v / v0:  v0 > 0: vx' = (cd*vx - sd*vy)*f, vy' = (sd*vx + cd*vy)*f;
+                  v0 = 0 and v > 0: (vx', vy') = v*(cos h', sin h'); otherwise unchanged.  The other velocity
+                  components are unchanged.  A VEHICLE / PID slot's controller speed is v.
+     So a component whose sigma is 0 is bit-identical to the unperturbed reset.  The RSS pass and the ego
+     metrics of the reset see the perturbed start.  The reset does not test collisions (as sg_reset): a
+     perturbed box that overlaps another collides at the first tick.
+   - The caller's obligation: with kind_mask {VEHICLE[,EMPTY]} every vehicle slot must be present at T.
+   init non-NULL, sigma finite and >= 0, counter non-NULL.  Other scenarios are left as sg_reset_scenarios
+   leaves them. */
+int sg_reset_scenarios_init(const SgScene* scene, const SgParams* params, SgState* state, const uint8_t* mask,
+                            const SgResetInit* init, int device, void* stream);
 
 /* Observations of the agents of SgEnvSpec (see there) for the scenarios with mask[n] != 0 (NULL: all):
    obs [N][A][F] fp32 (computed in fp64, rounded once), agent_mask [N][A] (the slot exists and is present),

@@ -11,7 +11,7 @@ import math
 import os
 from typing import Dict, Optional
 
-ABI_VERSION = 17
+ABI_VERSION = 18
 
 # SgKind
 KIND_EMPTY, KIND_REPLAY, KIND_AGENT_REPLAY, KIND_VEHICLE, KIND_PEDESTRIAN, KIND_HOST, KIND_PID = range(7)
@@ -247,6 +247,47 @@ class SgEnvSpec(C.Structure):
     ]
 
 
+class SgResetInit(C.Structure):
+    _fields_ = [
+        ("t_start", _p),
+        ("start_window", _p),
+        ("counter", _p),
+        ("perturb", _p),
+        ("sigma", C.c_double * 4),
+        ("seed", C.c_uint64),
+    ]
+
+
+def start_windows(scene, persist: bool, min_remaining: float):
+    """
+    [N] fp64, computed on the host from a lowered scene (``PackedScene``): for scenario n the largest w >= 0 with
+    t0 + w <= length - min_remaining such that every VEHICLE / PID slot present at t0 stays present over
+    [t0, t0 + w], i.e. its last control point is >= t0 + w (static slots, with one row, and every slot under
+    ``persist`` stay present anyway).  So a reset at any start in [t0, t0 + w] keeps the vehicles present (the
+    promise of SgScene.kind_mask) and leaves at least ``min_remaining`` seconds of the log.
+    """
+    import numpy as np
+
+    N, M = scene.N, scene.M
+    t0 = np.asarray(scene.t0, np.float64)
+    w = np.asarray(scene.length, np.float64) - float(min_remaining) - t0
+    if not persist:
+        kind = np.asarray(scene.kind).reshape(N * M)
+        off = np.asarray(scene.traj_off, np.int64)
+        rows = np.asarray(scene.traj_rows, np.float64).reshape(-1, 7)
+        K = off[1:] - off[:-1]
+        ctl = ((kind == KIND_VEHICLE) | (kind == KIND_PID)) & (K > 1)
+        idx = np.nonzero(ctl)[0]
+        first, last = rows[off[idx], 0], rows[off[idx + 1] - 1, 0]
+        n = idx // M
+        # present at t0 (within its logged span): bounded by its last control point
+        here = (first <= t0[n]) & (t0[n] <= last)
+        lim = np.full(N, np.inf)
+        np.minimum.at(lim, n[here], last[here] - t0[n[here]])
+        w = np.minimum(w, lim)
+    return np.maximum(w, 0.0)
+
+
 # number of reward terms of sg_env_reward: progress, collision, off_road, tracking, rss
 ENV_TERMS = ("progress", "collision", "off_road", "tracking", "rss")
 
@@ -454,6 +495,7 @@ EXPORTS = [
     "abi_version", "sizeof", "last_error", "default_params", "reset", "rollout",
     "test_box_pairs", "future_collisions", "fill_random_actions", "rollout_host", "host_h2d_bytes",
     "host_d2h_bytes", "reset_scenarios", "env_observe", "env_reward", "fork_state", "plan_sample", "plan_update",
+    "reset_scenarios_init",
 ]
 
 
@@ -499,6 +541,10 @@ def bind(lib: C.CDLL, prefix: str) -> Dict[str, object]:
     get("plan_update", C.c_int,
         [C.POINTER(SgEnvSpec), C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, _p, _p, C.c_int, _p, _p, C.c_int,
          _p, _p, _p, C.c_int, _p], required=False)
+    # sg_reset_scenarios_init: the product exports it; its oracle is test code (tests/reset_oracle.c)
+    get("reset_scenarios_init", C.c_int,
+        [C.POINTER(SgScene), C.POINTER(SgParams), C.POINTER(SgState), _p, C.POINTER(SgResetInit), C.c_int, _p],
+        required=False)
     get("rollout", C.c_int,
         [C.POINTER(SgScene), C.POINTER(SgParams), C.POINTER(SgState), C.POINTER(SgInputs),
          C.c_int, C.c_int, _p])
@@ -525,6 +571,8 @@ def bind(lib: C.CDLL, prefix: str) -> Dict[str, object]:
     structs = [SgParams, SgScene, SgState, SgInputs, SgEvent, SgActionRng, SgHostResults]
     if "env_observe" in f:  # (a library that takes SgEnvSpec knows its size)
         structs.append(SgEnvSpec)
+        if "reset_scenarios_init" in f:
+            structs.append(SgResetInit)
     for which, st in enumerate(structs):
         if f["sizeof"](which) != C.sizeof(st):
             raise RuntimeError(

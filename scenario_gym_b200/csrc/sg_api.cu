@@ -44,7 +44,8 @@ static int check_rng(const SgActionRng& r) {
 }
 
 static int launch(const SgScene* sc, const SgParams* p, SgState* st, const SgInputs* in, int n_ticks,
-                  int device, void* stream, int reset, const uint8_t* reset_mask = nullptr) {
+                  int device, void* stream, int reset, const uint8_t* reset_mask = nullptr,
+                  const SgResetInit* reset_init = nullptr) {
   if (!sc || !p || !st) return set_msg("null argument");
   if (sc->n_slots < 1 || sc->n_slots > 1024) return set_msg("n_slots must be in 1..1024");
   if (sc->n_scenarios < 1) return set_msg("n_scenarios must be >= 1");
@@ -79,7 +80,7 @@ static int launch(const SgScene* sc, const SgParams* p, SgState* st, const SgInp
   if (smem > 227 * 1024) return set_msg("scenario does not fit in shared memory");
   cudaStream_t s = (cudaStream_t)stream;
   if (reset) {
-    err = sgi_launch_reset(rss, big, blocks, threads, smem, s, *sc, *p, *st, L, reset_mask);
+    err = sgi_launch_reset(rss, big, blocks, threads, smem, s, *sc, *p, *st, L, reset_mask, reset_init);
     if (err != cudaSuccess) return set_err("sg_reset_kernel launch", err);
     return 0;
   }
@@ -143,6 +144,7 @@ int64_t sg_sizeof(int which) {
     case 5: return sizeof(SgActionRng);
     case 6: return sizeof(SgHostResults);
     case 7: return sizeof(SgEnvSpec);
+    case 8: return sizeof(SgResetInit);
   }
   return -1;
 }
@@ -200,6 +202,16 @@ int sg_rollout(const SgScene* scene, const SgParams* params, SgState* state, con
 int sg_reset_scenarios(const SgScene* scene, const SgParams* params, SgState* state, const uint8_t* mask,
                        int device, void* stream) {
   return launch(scene, params, state, nullptr, 0, device, stream, 1, mask);
+}
+
+int sg_reset_scenarios_init(const SgScene* scene, const SgParams* params, SgState* state, const uint8_t* mask,
+                            const SgResetInit* init, int device, void* stream) {
+  if (!init) return set_msg("null argument");
+  for (int c = 0; c < 4; ++c)
+    if (!isfinite(init->sigma[c]) || init->sigma[c] < 0.0)
+      return set_msg("sg_reset_scenarios_init: sigma must be finite and >= 0");
+  if (!init->counter) return set_msg("sg_reset_scenarios_init: counter missing");
+  return launch(scene, params, state, nullptr, 0, device, stream, 1, mask, init);
 }
 
 // the checks sg_env_observe and sg_env_reward share; `view` gets the scene with its plane stride stated

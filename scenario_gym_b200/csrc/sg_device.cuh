@@ -419,8 +419,12 @@ SG_DEV uint64_t sg_splitmix64(uint64_t z) {
   z = (z ^ (z >> 27)) * 0x94D049BB133111EBULL;
   return z ^ (z >> 31);
 }
+// the stream's first splitmix64 value for the key (seed, i, tick)
+SG_DEV uint64_t sg_noise_key(uint64_t seed, int64_t i, int tick) {
+  return sg_splitmix64(seed ^ sg_splitmix64((uint64_t)i * 0x9E3779B97F4A7C15ULL + (uint64_t)(unsigned)tick));
+}
 static __device__ __noinline__ double2 sg_noise2(uint64_t seed, int64_t i, int tick) {
-  const uint64_t a = sg_splitmix64(seed ^ sg_splitmix64((uint64_t)i * 0x9E3779B97F4A7C15ULL + (uint64_t)(unsigned)tick));
+  const uint64_t a = sg_noise_key(seed, i, tick);
   const uint64_t b = sg_splitmix64(a);
   const double u1 = ((double)(a >> 11) + 1.0) * (1.0 / 9007199254740992.0);  // (0, 1]
   const double u2 = (double)(b >> 11) * (1.0 / 9007199254740992.0);          // [0, 1)
@@ -428,4 +432,8 @@ static __device__ __noinline__ double2 sg_noise2(uint64_t seed, int64_t i, int t
   double sn, cs;
   sincos(2.0 * M_PI * u2, &sn, &cs);
   return make_double2(r * cs, r * sn);
+}
+// a uniform in [0, 1) from the same key: (a >> 11) * 2^-53, a the value sg_noise2 starts from
+SG_DEV double sg_uniform(uint64_t seed, int64_t i, int tick) {
+  return (double)(sg_noise_key(seed, i, tick) >> 11) * (1.0 / 9007199254740992.0);
 }

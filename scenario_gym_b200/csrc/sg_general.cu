@@ -5,6 +5,8 @@
 #include "sg_internal.h"
 #include "sg_pcg.cuh"
 
+#include <string.h>
+
 // ---------------------------------------------------------------------------------
 // General scenes: replay / batch replay / vehicles / pedestrians / host-driven slots.
 // ---------------------------------------------------------------------------------
@@ -353,12 +355,60 @@ sg_rollout_kernel(SgScene sc, SgParams p, SgState st, SgInputs in, int n_ticks, 
   store_cold(st, c, n, s, W, ego_slot);
 }
 
+// sg_reset_scenarios_init (include/sg_b200.h): the start time of scenario n and the draw's tick value 2k
+SG_DEV int reset_tick2(const SgResetInit& init, int n) { return (int)(uint32_t)((uint64_t)init.counter[n] * 2u); }
+SG_DEV double reset_start_time(const SgScene& sc, const SgResetInit& init, int n) {
+  if (init.t_start) return init.t_start[n];
+  if (!init.start_window) return sc.t0[n];
+  const double u = sg_uniform(init.seed, -1 - ((int64_t)n + sc.scenario_base), reset_tick2(init, n));
+  return sc.t0[n] + u * init.start_window[n];
+}
+// the perturbed start of a present slot with noise counter `ctr`; returns the speed v
+SG_DEV double perturb_start(const SgResetInit& init, int64_t ctr, int tick2, double pose[6], double vel[6]) {
+  const double* sg = init.sigma;
+  const double2 z01 = sg_noise2(init.seed, ctr, tick2), z23 = sg_noise2(init.seed, ctr, tick2 + 1);
+  const double v0 = norm2(vel[0], vel[1]);
+  double v = v0;
+  if (sg[0] != 0.0 || sg[1] != 0.0) {
+    double sh, ch;
+    sincos(pose[3], &sh, &ch);
+    const double lon = sg[0] * z01.x, lat = sg[1] * z01.y;
+    pose[0] = pose[0] + (ch * lon - sh * lat);
+    pose[1] = pose[1] + (sh * lon + ch * lat);
+  }
+  double dh = 0.0;
+  if (sg[2] != 0.0) {
+    dh = sg[2] * z23.x;
+    pose[3] = pose[3] + dh;
+  }
+  if (sg[2] != 0.0 || sg[3] != 0.0) {
+    v = v0 + sg[3] * z23.y;
+    v = v > 0.0 ? v : 0.0;
+    if (v0 > 0.0) {
+      double sd, cd;
+      sincos(dh, &sd, &cd);
+      const double f = v / v0, vx = vel[0], vy = vel[1];
+      vel[0] = (cd * vx - sd * vy) * f;
+      vel[1] = (sd * vx + cd * vy) * f;
+    } else if (v > 0.0) {
+      double sh, ch;
+      sincos(pose[3], &sh, &ch);
+      vel[0] = v * ch;
+      vel[1] = v * sh;
+    }
+  }
+  return v;
+}
+
 // State.reset(t0) + Agent/Metric/StateCallback resets (reference state/state.py:106-143,
 // controller.py:100-103, metrics/trajectory.py:13-18, metrics/rss/callback.py:44-55).
 // mask != NULL: only the scenarios with mask[n] != 0 (a whole group leaves, so its barriers stay matched)
-template <bool RSS, int MAXT>
+// INIT: sg_reset_scenarios_init -- the start time of `init` instead of t0, the flagged agents' starts perturbed
+// (include/sg_b200.h); the INIT = false instantiations do not read `init`.
+template <bool RSS, int MAXT, bool INIT>
 __global__ void __launch_bounds__(MAXT, MAXT >= 1024 ? 1 : 2)
-sg_reset_kernel(SgScene sc, SgParams p, SgState st, GroupLayout L, const uint8_t* __restrict__ mask) {
+sg_reset_kernel(SgScene sc, SgParams p, SgState st, GroupLayout L, const uint8_t* __restrict__ mask,
+                SgResetInit init) {
   extern __shared__ __align__(16) unsigned char smem[];
   const int G = L.G, M = sc.n_slots, W = L.W;
   const int gpb = blockDim.x / G;
@@ -374,7 +424,7 @@ sg_reset_kernel(SgScene sc, SgParams p, SgState st, GroupLayout L, const uint8_t
   const int64_t i = c.i, nm = c.nm;
   const int kind = live ? sc.kind[i] : SG_KIND_EMPTY;
   const int ego_slot = sc.ego_slot[n];
-  const double t = sc.t0[n];
+  const double t = INIT ? reset_start_time(sc, init, n) : sc.t0[n];  // (every thread of the group alike)
   double pose[6] = {0, 0, 0, 0, 0, 0}, vel[6] = {0, 0, 0, 0, 0, 0};
   double speed = 0;
   int orient_hint = 0;
@@ -396,6 +446,10 @@ sg_reset_kernel(SgScene sc, SgParams p, SgState st, GroupLayout L, const uint8_t
       for (int f = 0; f < 6; ++f) pose[f] = 0.0;
     }
     if (kind == SG_KIND_VEHICLE || kind == SG_KIND_PID) speed = norm2(vel[0], vel[1]);  // controller.py:100-103
+    if (INIT && present && init.perturb && init.perturb[i]) {
+      const double v = perturb_start(init, ((int64_t)n + sc.scenario_base) * M + s, reset_tick2(init, n), pose, vel);
+      if (kind == SG_KIND_VEHICLE || kind == SG_KIND_PID) speed = v;
+    }
   }
   uint8_t rss_state = 0, rss_last = SG_RSS_NONE;
   double sd[2] = {0.0, 0.0}, ratio[2] = {INFINITY, INFINITY};  // callback.py:51-55
@@ -461,16 +515,16 @@ sg_reset_kernel(SgScene sc, SgParams p, SgState st, GroupLayout L, const uint8_t
   if (s < W) st.ego_hits[(int64_t)n * W + s] = 0;
 }
 
-template <bool RSS>
+template <bool RSS, bool INIT>
 static cudaError_t launch_reset_t(bool big, int blocks, int threads, size_t smem, cudaStream_t s,
                                 const SgScene& sc, const SgParams& p, const SgState& st,
-                                const GroupLayout& L, const uint8_t* mask) {
-  auto kern = big ? sg_reset_kernel<RSS, 1024> : sg_reset_kernel<RSS, SG_THREADS>;
+                                const GroupLayout& L, const uint8_t* mask, const SgResetInit& init) {
+  auto kern = big ? sg_reset_kernel<RSS, 1024, INIT> : sg_reset_kernel<RSS, SG_THREADS, INIT>;
   if (smem > 48 * 1024) {
     cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (err != cudaSuccess) return err;
   }
-  kern<<<blocks, threads, smem, s>>>(sc, p, st, L, mask);
+  kern<<<blocks, threads, smem, s>>>(sc, p, st, L, mask, init);
   return cudaGetLastError();
 }
 
@@ -489,9 +543,13 @@ static cudaError_t launch_rollout_t(bool big, int blocks, int threads, size_t sm
 
 cudaError_t sgi_launch_reset(bool rss, bool big, int blocks, int threads, size_t smem, cudaStream_t s,
                              const SgScene& sc, const SgParams& p, const SgState& st, const GroupLayout& L,
-                             const uint8_t* mask) {
-  return rss ? launch_reset_t<true>(big, blocks, threads, smem, s, sc, p, st, L, mask)
-             : launch_reset_t<false>(big, blocks, threads, smem, s, sc, p, st, L, mask);
+                             const uint8_t* mask, const SgResetInit* init) {
+  if (init) return rss ? launch_reset_t<true, true>(big, blocks, threads, smem, s, sc, p, st, L, mask, *init)
+                       : launch_reset_t<false, true>(big, blocks, threads, smem, s, sc, p, st, L, mask, *init);
+  SgResetInit none;
+  memset(&none, 0, sizeof(none));
+  return rss ? launch_reset_t<true, false>(big, blocks, threads, smem, s, sc, p, st, L, mask, none)
+             : launch_reset_t<false, false>(big, blocks, threads, smem, s, sc, p, st, L, mask, none);
 }
 
 cudaError_t sgi_launch_rollout(bool ped, bool rss, bool big, int blocks, int threads, size_t smem,

@@ -7,10 +7,11 @@
 #include "sg_layout.h"
 #include "sg_pcg.cuh"
 
-// mask: [N] scenarios to reset (NULL: all)
+// mask: [N] scenarios to reset (NULL: all); init: the start times / perturbation of sg_reset_scenarios_init
+// (NULL: the reset at t0, sg_reset_scenarios)
 cudaError_t sgi_launch_reset(bool rss, bool big, int blocks, int threads, size_t smem, cudaStream_t s,
                              const SgScene& sc, const SgParams& p, const SgState& st, const GroupLayout& L,
-                             const uint8_t* mask);
+                             const uint8_t* mask, const SgResetInit* init);
 cudaError_t sgi_launch_rollout(bool ped, bool rss, bool big, int blocks, int threads, size_t smem,
                                cudaStream_t s, const SgScene& sc, const SgParams& p, const SgState& st,
                                const SgInputs& in, const SgRngDev& rng, int n_ticks, const GroupLayout& L);

@@ -133,12 +133,19 @@ class Engine:
         return int(sum(t.numel() * t.element_size() for t in self._state_t.values()))
 
     # ------------------------------------------------------------------ API
-    def reset(self, mask: Optional[torch.Tensor] = None) -> None:
+    def reset(self, mask: Optional[torch.Tensor] = None, init: Optional[abi.SgResetInit] = None) -> None:
         """
         State.reset + metric/controller resets for every scenario (sg_reset), or -- ``mask``: a uint8 / bool
         device tensor [N] -- for the scenarios with ``mask[n] != 0`` only (sg_reset_scenarios; the other
-        scenarios and the event count are left as they are).
+        scenarios and the event count are left as they are).  ``init``: the start times and perturbation of
+        sg_reset_scenarios_init (its device arrays are the caller's), for the masked scenarios or, without a
+        mask, for all of them (the event count is then left as it is too).
         """
+        if init is not None:
+            m = None if mask is None else self._scenario_mask(mask).data_ptr()
+            self._check(self.lib["reset_scenarios_init"](C.byref(self._sc), C.byref(self.params), C.byref(self._st),
+                                                         m, C.byref(init), self.dev_index, self._stream()))
+            return
         if mask is None:
             self._check(self.lib["reset"](C.byref(self._sc), C.byref(self.params), C.byref(self._st),
                                           self.dev_index, self._stream()))

@@ -2,9 +2,9 @@
 ``VecScenarioEnv`` -- a closed-loop, batched environment on the device: a policy chooses every step's
 VehicleActions from observations, and observations, rewards, termination and the reset of finished
 scenarios are all computed by the library's kernels (``sg_env_observe``, ``sg_env_reward``,
-``sg_reset_scenarios``; semantics in ``include/sg_b200.h``).  ``step()`` and ``reset()`` enqueue their work
-on the current CUDA stream with no per-scenario Python and no device -> host synchronisation; every buffer
-is allocated once, when the env is built.
+``sg_reset_scenarios`` / ``sg_reset_scenarios_init``; semantics in ``include/sg_b200.h``).  ``step()`` and
+``reset()`` enqueue their work on the current CUDA stream with no per-scenario Python and no device -> host
+synchronisation; every buffer is allocated once, when the env is built.
 """
 from __future__ import annotations
 
@@ -55,6 +55,33 @@ class ObsSpec:
                                   int(self.lidar_rays), int(self.map_edges))
 
 
+@dataclass
+class ResetSpec:
+    """Randomised episode starts of a ``VecScenarioEnv`` (include/sg_b200.h, sg_reset_scenarios_init).  Every
+    reset, the auto-reset in ``step()`` included, starts scenario n at t0 + u * window[n], u uniform in [0, 1),
+    window[n] = min(``start_offset``, ``env.start_window[n]``): the longest delay that keeps every vehicle of the
+    log present and leaves ``min_remaining`` seconds of it.  Each agent's start is then moved by N(0, std)
+    noise: ``lon`` / ``lat`` metres along / across its heading, ``heading`` radians and ``speed`` m/s (the speed
+    is kept >= 0 and the velocity turns with the heading).  The draws are a pure function of ``seed``, the
+    scenario, the agent and the scenario's episode count, so a seeded sequence of episodes repeats.  A start
+    whose box overlaps another entity's collides at the first tick; nothing rejects it."""
+    start_offset: float = 0.0
+    min_remaining: float = 1.0
+    lon: float = 0.0
+    lat: float = 0.0
+    heading: float = 0.0
+    speed: float = 0.0
+    seed: int = 0
+
+    def __post_init__(self):
+        for name in ("start_offset", "min_remaining", "lon", "lat", "heading", "speed"):
+            v = getattr(self, name)
+            if isinstance(v, bool) or not isinstance(v, (int, float)) or not (math.isfinite(v) and v >= 0.0):
+                raise ValueError(f"ResetSpec.{name} must be a finite number >= 0, got {v!r}")
+        if isinstance(self.seed, bool) or not isinstance(self.seed, (int, np.integer)):
+            raise ValueError(f"ResetSpec.seed must be an int, got {self.seed!r}")
+
+
 def _ego_policy(scenario: Scenario, entity: Entity):
     """Default ``create_agent`` of the env: the ego is driven by the policy, everything else is replayed."""
     return PolicyAgent(entity) if entity is scenario.ego else None
@@ -77,13 +104,21 @@ class VecScenarioEnv:
     finishes is reset in the same step: ``obs`` holds the first observation of its next episode,
     ``info["final_obs"]`` the observation it finished with, ``info["final"]`` its episode results (rows of
     scenarios that did not finish hold their running values).
+
+    ``reset_spec`` (a ``ResetSpec``): every reset, the auto-reset included, starts at a drawn time inside the log
+    with the agents' starts perturbed (``sg_reset_scenarios_init``); ``start_window`` [N] fp64 holds the longest
+    delay after t0 each scenario allows (every vehicle of the log still present, ``min_remaining`` seconds left).
+    A pedestrian starting later restarts at the first point of its route, as at t0: routes are not re-targeted.
     """
 
     def __init__(self, scenarios: List[Scenario], create_agent: Callable = _ego_policy,
                  timestep: float = 1.0 / 30.0, terminal_conditions: Optional[List[Union[str, Callable]]] = None,
                  state_callbacks: Optional[List[StateCallback]] = None, obs: Optional[ObsSpec] = None,
                  reward_weights: Optional[Union[Mapping[str, float], Sequence[float]]] = None,
-                 device: Union[int, str, torch.device] = 0, record: bool = False):
+                 device: Union[int, str, torch.device] = 0, record: bool = False,
+                 reset_spec: Optional[ResetSpec] = None):
+        if reset_spec is not None and not isinstance(reset_spec, ResetSpec):
+            raise ValueError(f"reset_spec must be a ResetSpec or None, got {type(reset_spec).__name__}")
         if record:
             raise NotImplementedError("VecScenarioEnv keeps no pose trace (record=True needs ScenarioGym)")
         terminal_conditions = ["max_length"] if terminal_conditions is None else list(terminal_conditions)
@@ -194,6 +229,28 @@ class VecScenarioEnv:
         self._spec = spec
         self._info = {"agent_mask": self._agent_mask, "episode_step": eng.tensor("tick"), "episode": self._episode}
 
+        # episode starts (sg_reset_scenarios_init): the valid windows are decided once, on the host
+        self.reset_spec = reset_spec
+        rs = reset_spec if reset_spec is not None else ResetSpec()
+        win = abi.start_windows(eng.scene, bool(eng.params.persist), rs.min_remaining)
+        self.start_window = torch.from_numpy(win).to(dev)
+        self._draw_window = torch.from_numpy(np.minimum(win, float(rs.start_offset))).to(dev)
+        self._t_start = zeros(N, dtype=torch.float64)
+        self._counter = zeros(N, dtype=torch.int64)
+        perturb = np.zeros(N * M, np.uint8)
+        perturb[dst] = 1
+        self._perturb = torch.from_numpy(perturb).to(dev)
+        self._init = abi.SgResetInit()  # draws the start (reset() and step())
+        self._init.start_window = self._draw_window.data_ptr()
+        self._init.counter = self._counter.data_ptr()
+        if reset_spec is not None:
+            self._init.perturb = self._perturb.data_ptr()
+            for k, v in enumerate((rs.lon, rs.lat, rs.heading, rs.speed)):
+                self._init.sigma[k] = float(v)
+        self._init.seed = int(rs.seed) & (2**64 - 1)
+        self._init_at = abi.SgResetInit.from_buffer_copy(self._init)  # starts at the times of reset(start_time)
+        self._init_at.t_start = self._t_start.data_ptr()
+
     # ------------------------------------------------------------------ API
     def agent_entities(self, n: int) -> List[Entity]:
         """The entities behind agents 0 .. of scenario ``n`` (shorter than ``A`` where the row is padded)."""
@@ -213,10 +270,39 @@ class VecScenarioEnv:
         allocated here, once."""
         return MPPIPlanner(self, B, H, sigma, temperature, iterations, seed)
 
-    def reset(self) -> Tuple[torch.Tensor, Dict[str, torch.Tensor]]:
-        """Every scenario back to its start (sg_reset) and observed; episode counters restart at 0."""
+    def reset(self, seed: Optional[int] = None, start_time: Optional[torch.Tensor] = None
+              ) -> Tuple[torch.Tensor, Dict[str, torch.Tensor]]:
+        """
+        Every scenario back to its start and observed; episode counters restart at 0.  Without a ``ResetSpec``
+        the start is the log's (sg_reset), with one it is drawn as the spec says.  ``seed``: the draws' seed from
+        now on, with every scenario's draw count back at 0, so the same seed replays the same episodes.
+        ``start_time`` (fp64 [N] on the env's device, with or without a spec): start scenario n that many seconds
+        after its t0, clamped on the device to [0, ``start_window[n]``] (NaN counts as 0); a spec's perturbation
+        still applies.
+        """
         eng = self._engine
-        eng.reset()
+        if seed is not None:
+            if isinstance(seed, bool) or not isinstance(seed, (int, np.integer)):
+                raise ValueError(f"seed must be an int, got {seed!r}")
+            self._init.seed = self._init_at.seed = int(seed) & (2**64 - 1)
+            self._counter.zero_()
+        if start_time is not None:
+            if not isinstance(start_time, torch.Tensor) or tuple(start_time.shape) != (self.N,) \
+                    or start_time.dtype != torch.float64 or start_time.device != self.device:
+                raise ValueError(f"start_time must be a float64 tensor of shape ({self.N},) on {self.device}")
+            torch.nan_to_num(start_time, nan=0.0, out=self._t_start)
+            torch.clamp(self._t_start, min=0.0, out=self._t_start)
+            torch.minimum(self._t_start, self.start_window, out=self._t_start)
+            self._t_start.add_(eng._scene_t["t0"])
+            init = self._init_at
+        else:
+            init = self._init if self.reset_spec is not None else None
+        if init is None:
+            eng.reset()
+        else:
+            eng.reset(init=init)
+            eng.tensor("event_count").zero_()  # (as sg_reset)
+            self._counter.add_(1)
         self._episode.zero_()
         self._resets += 1  # (a planner cannot see this reset in the episode counters when they were 0)
         eng.env_observe(self._spec, self._obs, self._agent_mask)
@@ -246,7 +332,11 @@ class VecScenarioEnv:
         for k, f in _FINAL_FIELDS.items():
             self._final[k].copy_(eng.tensor(f))
         torch.bitwise_or(self._terminated, self._truncated, out=self._finished)
-        eng.reset(mask=self._finished)
+        if self.reset_spec is None:
+            eng.reset(mask=self._finished)
+        else:
+            eng.reset(mask=self._finished, init=self._init)
+            self._counter.add_(self._finished)
         eng.env_observe(self._spec, self._obs, self._agent_mask, mask=self._finished)
         self._episode.add_(self._finished)
         eng.tensor("event_count").zero_()  # ego collision events are not kept across steps

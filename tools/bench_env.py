@@ -2,8 +2,8 @@
 """
 bench_env.py -- throughput of the closed-loop environment (VecScenarioEnv) and where its step goes.
 
-    python tools/bench_env.py [--out FILE] [--lidar R] [--map Km]   # one JSON line per workload on stdout (and
-                                                                     # appended to FILE)
+    python tools/bench_env.py [--out FILE] [--lidar R] [--map Km] [--reset]   # one JSON line per workload on
+                                                                               # stdout (and appended to FILE)
 
 Workloads:
   vehicles  12 500 scenarios x 64 VehicleController entities (synthetic.vehicles_config, 625 distinct
@@ -30,6 +30,12 @@ Reported per workload:
   map_us / map_brute_us                 the map kernel's time per observe (observe with the map block minus observe
                                         without it, CUDA events over 50 calls each), with the env's culling grid and
                                         with the same table built as a single cell (brute force, same kernel)
+  reset_{full,1pct}_{plain,init}_us     with --reset (the envs are then built with RESET_SPEC: randomised starts
+                                        and perturbed agents): the masked reset's device time (CUDA events over 20
+                                        calls) with every scenario / every 100th selected, through the plain kernel
+                                        (sg_reset_scenarios) and the init kernel (sg_reset_scenarios_init)
+  env_steps_per_s_spec / _plain         with --reset: step() + policy with the spec's auto-reset, and with the plain
+                                        one (env.reset_spec = None), host clock over >= 1 s each
   device / power_limit_w                the card and its power limit
 """
 from __future__ import annotations
@@ -51,7 +57,7 @@ import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 from scenario_gym_b200 import (BoundingBox, CatalogEntry, Entity, ObsSpec, Pedestrian, PolicyAgent,  # noqa: E402
-                               Scenario, Trajectory, VecScenarioEnv, Vehicle, abi, synthetic)
+                               ResetSpec, Scenario, Trajectory, VecScenarioEnv, Vehicle, abi, synthetic)
 from scenario_gym_b200.engine import Engine  # noqa: E402
 
 
@@ -61,7 +67,11 @@ def policy(obs):
                         torch.atan2(ty, tx).clamp(-0.7, 0.7)], -1)
 
 
-def vehicles_env(obs):
+# --reset: episodes start up to 2 s into the log with every agent's start perturbed
+RESET_SPEC = ResetSpec(start_offset=2.0, min_remaining=1.0, lon=0.5, lat=0.2, heading=0.05, speed=1.0, seed=0)
+
+
+def vehicles_env(obs, reset_spec=None):
     distinct, reps, M = 625, 20, 64
     cfg = synthetic.vehicles_config(seed=0, N=distinct, M=M, T=256)
     rows = synthetic.two_knot_rows(cfg).reshape(distinct, M, 2, 7)
@@ -69,10 +79,11 @@ def vehicles_env(obs):
     town = synthetic.grid_town(seed=0, half_extent=200.0) if obs.map_edges > 0 else None
     scs = [Scenario([Vehicle(ce, trajectory=Trajectory(rows[n, m]), ref="ego" if m == 0 else f"entity_{m}")
                      for m in range(M)], road_network=town) for n in range(distinct)]
-    return VecScenarioEnv(scs * reps, create_agent=lambda s, e: PolicyAgent(e), timestep=cfg.dt, obs=obs)
+    return VecScenarioEnv(scs * reps, create_agent=lambda s, e: PolicyAgent(e), timestep=cfg.dt, obs=obs,
+                          reset_spec=reset_spec)
 
 
-def xosc_env(obs):
+def xosc_env(obs, reset_spec=None):
     sys.path.insert(0, os.path.join(REPO, "tests"))
     from helpers import golden, manifest, sub
 
@@ -94,7 +105,7 @@ def xosc_env(obs):
         town = synthetic.grid_town(seed=0, half_extent=float((hi - lo).max()) / 2 + 20.0, center=(lo + hi) / 2)
         for sc in scs:
             sc.road_network = town
-    return VecScenarioEnv([scs[k % len(scs)] for k in range(4096)], obs=obs)
+    return VecScenarioEnv([scs[k % len(scs)] for k in range(4096)], obs=obs, reset_spec=reset_spec)
 
 
 def card():
@@ -180,6 +191,7 @@ def measure(name, env):
     assert int(fused.get("tick").min()) == 64, "every scenario must run the 64 timed ticks"
     del fused
     maps = map_times(env) if env.obs_spec.map_edges > 0 else {}
+    resets = reset_times(env) if env.reset_spec is not None else {}
     F = env.n_features
     obs_bytes = env.N * env.A * (4 * F + 1 + 9) + env.N * 9
     dev, power = card()
@@ -194,7 +206,7 @@ def measure(name, env):
         "observe_bytes": obs_bytes, "observe_GBps": obs_bytes / (acc["observe"] * 1e-6) / 1e9,
         "lidar_rays": int(env.obs_spec.lidar_rays), "lidar_bytes": env.N * env.A * 4 * int(env.obs_spec.lidar_rays),
         "map_edges": int(env.obs_spec.map_edges), "map_bytes": env.N * env.A * 40 * int(env.obs_spec.map_edges),
-        **maps,
+        **maps, **resets,
         "library": os.path.basename(abi.PRODUCT_LIB),
         "device": dev, "power_limit_w": power,
     }
@@ -230,12 +242,62 @@ def map_times(env):
             "map_us": round(grid - base, 2), "map_brute_us": round(flat - base, 2)}
 
 
+def steps_per_s(env):
+    """step() + policy per second, host clock over >= 1 s ending in a synchronise (after 20 warm-up steps)."""
+    o, _ = env.reset()
+    for _ in range(20):
+        o, *_ = env.step(policy(o))
+    torch.cuda.synchronize()
+    steps, t0 = 0, time.perf_counter()
+    while True:
+        for _ in range(10):
+            o, *_ = env.step(policy(o))
+        steps += 10
+        torch.cuda.synchronize()
+        dt = time.perf_counter() - t0
+        if dt >= 1.0:
+            return steps / dt
+
+
+def reset_times(env):
+    """The masked reset's device time through the plain and the init kernel, for a full and a 1 % mask, and the
+    env's steps per second with its spec and with the plain auto-reset."""
+    eng, stream = env._engine, torch.cuda.current_stream()
+    n = torch.arange(env.N, device=env.device)
+    masks = {"full": torch.ones(env.N, dtype=torch.uint8, device=env.device),
+             "1pct": (n % 100 == 0).to(torch.uint8)}
+
+    def reset_us(mask, init, reps=20):
+        for _ in range(3):
+            eng.reset(mask=mask, init=init)
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record(stream)
+        for _ in range(reps):
+            eng.reset(mask=mask, init=init)
+        e1.record(stream)
+        torch.cuda.synchronize()
+        return round(e0.elapsed_time(e1) * 1e3 / reps, 2)
+
+    out = {"reset_spec": {k: getattr(env.reset_spec, k) for k in ("start_offset", "min_remaining", "lon", "lat",
+                                                                   "heading", "speed")}}
+    for k, m in masks.items():
+        out[f"reset_{k}_plain_us"] = reset_us(m, None)
+        out[f"reset_{k}_init_us"] = reset_us(m, env._init)
+    spec = env.reset_spec
+    out["env_steps_per_s_spec"] = steps_per_s(env)
+    env.reset_spec = None  # (the env's plain auto-reset: sg_reset_scenarios)
+    out["env_steps_per_s_plain"] = steps_per_s(env)
+    env.reset_spec = spec
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     ap.add_argument("--out", default=None, help="also append the JSON lines to this file")
     ap.add_argument("--workloads", default="vehicles,xosc")
     ap.add_argument("--lidar", type=int, default=0, help="lidar rays R of the observation (0: no lidar block)")
     ap.add_argument("--map", type=int, default=0, help="map edges Km of the observation (0: no town, no map block)")
+    ap.add_argument("--reset", action="store_true", help="build the envs with RESET_SPEC and time the resets")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("bench_env.py measures the GPU engine: no CUDA device")
@@ -243,7 +305,7 @@ def main():
                   map_edges=args.map, map_radius=50.0)
     for w in args.workloads.split(","):
         t0 = time.time()
-        env = {"vehicles": vehicles_env, "xosc": xosc_env}[w](obs)
+        env = {"vehicles": vehicles_env, "xosc": xosc_env}[w](obs, RESET_SPEC if args.reset else None)
         build_s = time.time() - t0
         rec = measure(w, env)
         rec["build_s"] = round(build_s, 1)
