@@ -45,7 +45,7 @@
 extern "C" {
 #endif
 
-#define SG_ABI_VERSION 18
+#define SG_ABI_VERSION 19
 
 /* entity slot kinds (who produces the slot's next pose each tick) */
 enum SgKind {
@@ -407,9 +407,55 @@ typedef struct SgEnvSpec {
   const int32_t* map_cell_edge;  /* edge indices e within the network, ascending per cell */
 } SgEnvSpec;
 
+/* Bird's-eye raster of each agent of SgEnvSpec (sg_env_raster): uint8 [C = 5][S][S] per agent, values 0 / 1.
+   S = size (pixels), res = resolution (metres per pixel), ahead = how far (metres) the raster's centre lies ahead
+   of the agent along its heading.  Pixel centres in the agent's frame (u forward, v to the left), h = 0.5 * res
+   (exact):  pu_i = ahead + (S - 1 - 2i) * h,  pv_j = (S - 1 - 2j) * h.  So row 0 lies furthest ahead, column 0
+   furthest left, and the image's "up" is the agent's heading.  (x, y, hd) is the agent's pose, (c, s) =
+   (cos hd, sin hd), rot as for the observation rows.  Every formula below is evaluated in fp64, in the operation
+   order written, with no FMA.
+     channels 0, 1, 2  driveable, walkable, impenetrable surface of network rn_of[n]: a pixel is set iff its centre
+                lies inside at least one polygon of that surface (an OR over polygons, never a parity over the whole
+                soup: lanes overlap their road).  Inside a polygon = crossing parity along the pixel's row over every
+                ring of the polygon, holes included: each vertex goes into the agent frame, a' = rot(ax - x, ay - y);
+                edge a -> b crosses row i iff (a'.u > pu_i) != (b'.u > pu_i), at
+                vc = a'.v + ((pu_i - a'.u) * (b'.v - a'.v)) / (b'.u - a'.u), and toggles pixel j iff vc > pv_j; the
+                pixel is inside iff it is toggled an odd number of times.  Away from the rings this agrees with the
+                strict containment of the reward's off_road term at the pixel's world centre; a centre on a ring
+                follows this half-open rule instead (a square aligned with the agent frame holds the centres on its
+                rear (least u) and right (least v) sides, not those on its front and left sides).  No network, or a surface without polygons: zeros.
+     channels 3, 4  the box of every other present slot j (j != the agent's slot): channel 4 the slots whose etype
+                is pedestrian, channel 3 every other one (vehicles, misc objects).  The box is the collision test's,
+                as the lidar defines it: centre (X, Y), axes (cj, sj), half extents hl, hw.  With the pixel's world
+                centre Px = x + (c*pu - s*pv), Py = y + (s*pu + c*pv), p = (Px - X, Py - Y),
+                ox = cj*px + sj*py, oy = -sj*px + cj*py, the pixel is set iff |ox| <= hl && |oy| <= hw (a closed set:
+                a box without area marks only the pixel centres exactly on it).
+   Absent and padding agents get an all-zero raster.
+   Culling (an implementation aid that must not change the result): with the raster's world centre
+   (x + c*ahead, y + s*ahead), its half-diagonal D = sqrt(2) * S * h and a margin m, a polygon may be skipped when
+   its bounding box widened by m misses the square of half-size D around that centre, and a box when its
+   circumscribed circle (radius sqrt(hl^2 + hw^2)) widened by m misses it; a row may test only the pixels near a
+   box's circle.  The exact predicates above decide every pixel that is tested.  Every pixel centre lies within
+   sqrt(2) * (S - 1) * h < D of the centre.  A polygon skipped this way lies, up to rounding, wholly outside the
+   square, so each row crosses each of its rings an even number of times with every crossing on the same side of
+   every pixel: it toggles nothing.  Rounding moves a transformed vertex, a crossing or a pixel's world centre by a
+   few ulps of the coordinates involved; m = 1e-9 x (1 + largest |coordinate| + D) (the polygons' coordinates for
+   SgRasterSpec.margin, the agent's and the box's for boxes, computed on the device) exceeds that by orders of
+   magnitude, as the map grid's margin does. */
+typedef struct SgRasterSpec {
+  int32_t size;             /* S: a multiple of 32 in 32..256 */
+  int32_t n_networks;       /* networks poly_box was built for: must be SgScene.n_networks */
+  double resolution;        /* metres per pixel, finite and > 0 */
+  double ahead;             /* metres, finite */
+  double margin;            /* m of the polygon culling (finite, >= 0): 1e-9 x (1 + largest |coordinate| + D) */
+  const double* poly_box;   /* [n_rn_polys][4] device: min x, min y, max x, max y of each polygon's edges;
+                               required when the scene has networks */
+} SgRasterSpec;
+
 int sg_abi_version(void);
 /* sizeof() of the ABI structs so bindings can verify their mirror: which = 0 SgParams,
-   1 SgScene, 2 SgState, 3 SgInputs, 4 SgEvent, 5 SgActionRng, 6 SgHostResults, 7 SgEnvSpec, 8 SgResetInit */
+   1 SgScene, 2 SgState, 3 SgInputs, 4 SgEvent, 5 SgActionRng, 6 SgHostResults, 7 SgEnvSpec, 8 SgResetInit,
+   9 SgRasterSpec */
 int64_t sg_sizeof(int which);
 const char* sg_last_error(void);
 void sg_default_params(SgParams* p);
@@ -470,6 +516,12 @@ int sg_reset_scenarios_init(const SgScene* scene, const SgParams* params, SgStat
    and the snapshot the next sg_env_reward compares against.  Rows of other scenarios are not written. */
 int sg_env_observe(const SgScene* scene, const SgParams* params, const SgState* state, const SgEnvSpec* spec,
                    const uint8_t* mask, float* obs, uint8_t* agent_mask, int device, void* stream);
+
+/* Bird's-eye rasters of the agents of SgEnvSpec (semantics at SgRasterSpec) for the scenarios with mask[n] != 0
+   (NULL: all): out [N][A][5][S][S] uint8, device memory, 16-byte aligned.  Rasters of other scenarios are not
+   written.  Reads the spec's agent_slot only: the observation blocks and the snapshot are not touched. */
+int sg_env_raster(const SgScene* scene, const SgParams* params, const SgState* state, const SgEnvSpec* spec,
+                  const SgRasterSpec* raster, const uint8_t* mask, uint8_t* out, int device, void* stream);
 
 /* Rewards of one environment step, after the tick and before any reset: reward [N][A], terms [N][A][5]
    (fp32).  For the scenarios whose done flag is set (an environment steps only scenarios that are not

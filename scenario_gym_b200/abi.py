@@ -11,7 +11,7 @@ import math
 import os
 from typing import Dict, Optional
 
-ABI_VERSION = 18
+ABI_VERSION = 19
 
 # SgKind
 KIND_EMPTY, KIND_REPLAY, KIND_AGENT_REPLAY, KIND_VEHICLE, KIND_PEDESTRIAN, KIND_HOST, KIND_PID = range(7)
@@ -258,6 +258,52 @@ class SgResetInit(C.Structure):
     ]
 
 
+class SgRasterSpec(C.Structure):
+    _fields_ = [
+        ("size", C.c_int32),
+        ("n_networks", C.c_int32),
+        ("resolution", C.c_double),
+        ("ahead", C.c_double),
+        ("margin", C.c_double),
+        ("poly_box", _p),
+    ]
+
+
+# the channels of sg_env_raster, in order
+RASTER_CHANNELS = ("driveable", "walkable", "impenetrable", "vehicles", "pedestrians")
+
+
+def raster_poly_boxes(rn_edge_off, rn_edges, half_diagonal: float):
+    """
+    ``SgRasterSpec.poly_box`` and ``margin`` of a scene's polygon soups (SgScene.rn_edge_off / rn_edges): [P, 4]
+    fp64 min x, min y, max x, max y over each polygon's edges (zeros for a polygon without edges, which toggles
+    nothing), and m = 1e-9 * (1 + largest |coordinate| + half_diagonal) (include/sg_b200.h, SgRasterSpec).
+    """
+    import numpy as np
+
+    off = np.asarray(rn_edge_off, np.int64)
+    edges = np.asarray(rn_edges, np.float64).reshape(-1, 4)
+    P = len(off) - 1
+    box = np.zeros((P, 4), np.float64)
+    if len(edges):
+        xs, ys = edges[:, 0::2], edges[:, 1::2]
+        lo_x, hi_x = xs.min(1), xs.max(1)
+        lo_y, hi_y = ys.min(1), ys.max(1)
+        full = off[1:] > off[:-1]
+        starts = off[:-1][full]
+        box[full, 0] = np.minimum.reduceat(lo_x, starts)
+        box[full, 1] = np.minimum.reduceat(lo_y, starts)
+        box[full, 2] = np.maximum.reduceat(hi_x, starts)
+        box[full, 3] = np.maximum.reduceat(hi_y, starts)
+    big = float(np.abs(edges).max()) if len(edges) else 0.0
+    return box, 1e-9 * (1.0 + big + float(half_diagonal))
+
+
+def raster_half_diagonal(size: int, resolution: float) -> float:
+    """The raster's half-diagonal sqrt(2) * S * h, h = resolution / 2 (the device's value)."""
+    return 1.4142135623730951 * (float(size) * (0.5 * float(resolution)))
+
+
 def start_windows(scene, persist: bool, min_remaining: float):
     """
     [N] fp64, computed on the host from a lowered scene (``PackedScene``): for scenario n the largest w >= 0 with
@@ -495,7 +541,7 @@ EXPORTS = [
     "abi_version", "sizeof", "last_error", "default_params", "reset", "rollout",
     "test_box_pairs", "future_collisions", "fill_random_actions", "rollout_host", "host_h2d_bytes",
     "host_d2h_bytes", "reset_scenarios", "env_observe", "env_reward", "fork_state", "plan_sample", "plan_update",
-    "reset_scenarios_init",
+    "reset_scenarios_init", "env_raster",
 ]
 
 
@@ -545,6 +591,10 @@ def bind(lib: C.CDLL, prefix: str) -> Dict[str, object]:
     get("reset_scenarios_init", C.c_int,
         [C.POINTER(SgScene), C.POINTER(SgParams), C.POINTER(SgState), _p, C.POINTER(SgResetInit), C.c_int, _p],
         required=False)
+    # sg_env_raster: the product exports it; its oracle is test code (tests/raster_oracle.c)
+    get("env_raster", C.c_int,
+        [C.POINTER(SgScene), C.POINTER(SgParams), C.POINTER(SgState), C.POINTER(SgEnvSpec), C.POINTER(SgRasterSpec),
+         _p, _p, C.c_int, _p], required=False)
     get("rollout", C.c_int,
         [C.POINTER(SgScene), C.POINTER(SgParams), C.POINTER(SgState), C.POINTER(SgInputs),
          C.c_int, C.c_int, _p])
@@ -573,6 +623,8 @@ def bind(lib: C.CDLL, prefix: str) -> Dict[str, object]:
         structs.append(SgEnvSpec)
         if "reset_scenarios_init" in f:
             structs.append(SgResetInit)
+            if "env_raster" in f:
+                structs.append(SgRasterSpec)
     for which, st in enumerate(structs):
         if f["sizeof"](which) != C.sizeof(st):
             raise RuntimeError(

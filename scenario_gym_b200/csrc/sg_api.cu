@@ -145,6 +145,7 @@ int64_t sg_sizeof(int which) {
     case 6: return sizeof(SgHostResults);
     case 7: return sizeof(SgEnvSpec);
     case 8: return sizeof(SgResetInit);
+    case 9: return sizeof(SgRasterSpec);
   }
   return -1;
 }
@@ -260,6 +261,30 @@ int sg_env_observe(const SgScene* scene, const SgParams* params, const SgState* 
   if (err != cudaSuccess) return set_err("cudaSetDevice", err);
   err = sgi_launch_env_observe((cudaStream_t)stream, view, *state, *spec, mask, obs, agent_mask);
   if (err != cudaSuccess) return set_err("sg_env_observe_kernel launch", err);
+  return 0;
+}
+
+int sg_env_raster(const SgScene* scene, const SgParams* params, const SgState* state, const SgEnvSpec* spec,
+                  const SgRasterSpec* raster, const uint8_t* mask, uint8_t* out, int device, void* stream) {
+  SgScene view;
+  int rc = check_env(scene, params, state, spec, &view);
+  if (rc) return rc;
+  if (!raster || !out) return set_msg("null argument");
+  if (raster->size < 32 || raster->size > 256 || raster->size % 32 != 0)
+    return set_msg("SgRasterSpec.size must be a multiple of 32 in 32..256");
+  if (!isfinite(raster->resolution) || !(raster->resolution > 0.0))
+    return set_msg("SgRasterSpec.resolution must be finite and > 0");
+  if (!isfinite(raster->ahead)) return set_msg("SgRasterSpec.ahead must be finite");
+  if (!isfinite(raster->margin) || raster->margin < 0.0)
+    return set_msg("SgRasterSpec.margin must be finite and >= 0");
+  if (raster->n_networks != scene->n_networks)
+    return set_msg("SgRasterSpec.n_networks differs from the scene's n_networks (poly_box is per polygon)");
+  if (scene->n_networks > 0 && !raster->poly_box) return set_msg("SgRasterSpec.poly_box missing (the scene has networks)");
+  if ((uintptr_t)out % 16 != 0) return set_msg("sg_env_raster: out must be 16-byte aligned");
+  cudaError_t err = cudaSetDevice(device);
+  if (err != cudaSuccess) return set_err("cudaSetDevice", err);
+  err = sgi_launch_env_raster((cudaStream_t)stream, view, *state, *spec, *raster, mask, out);
+  if (err != cudaSuccess) return set_err("sg_env_raster_kernel launch", err);
   return 0;
 }
 

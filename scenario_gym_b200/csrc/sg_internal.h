@@ -52,6 +52,9 @@ cudaError_t sgi_launch_env_observe(cudaStream_t s, const SgScene& sc, const SgSt
 cudaError_t sgi_launch_env_reward(cudaStream_t s, const SgScene& sc, const SgParams& p, const SgState& st,
                                   const SgEnvSpec& e, float* reward, float* terms, uint8_t* terminated,
                                   uint8_t* truncated);
+// sg_env_raster (sg_raster.cu); `sc` has its plane stride stated, the arguments are checked
+cudaError_t sgi_launch_env_raster(cudaStream_t s, const SgScene& sc, const SgState& st, const SgEnvSpec& e,
+                                  const SgRasterSpec& r, const uint8_t* mask, uint8_t* out);
 // sg_fork_state (sg_fork.cu); `sc` has its plane stride stated, the arguments are checked
 cudaError_t sgi_launch_fork(cudaStream_t s, const SgScene& sc, const SgState& src, SgState* const* dst, int n_dst,
                             const SgEnvSpec* src_spec, SgEnvSpec* const* dst_spec);

@@ -210,6 +210,20 @@ class Engine:
                                             C.byref(spec), None if m is None else m.data_ptr(), obs.data_ptr(),
                                             agent_mask.data_ptr(), self.dev_index, self._stream()))
 
+    def env_raster(self, spec: abi.SgEnvSpec, rspec: abi.SgRasterSpec, out: torch.Tensor,
+                   mask: Optional[torch.Tensor] = None) -> None:
+        """sg_env_raster into preallocated ``out`` (uint8 [N, A, 5, S, S], contiguous) for the scenarios of ``mask``
+        (None: all)."""
+        S = int(rspec.size)
+        if out.dtype != torch.uint8 or out.device != self.device or not out.is_contiguous() \
+                or tuple(out.shape) != (self.N, int(spec.n_agents), 5, S, S):
+            raise ValueError(f"out must be a contiguous uint8 tensor [{self.N}, {spec.n_agents}, 5, {S}, {S}] "
+                             f"on {self.device}")
+        m = None if mask is None else self._scenario_mask(mask)
+        self._check(self.lib["env_raster"](C.byref(self._sc), C.byref(self.params), C.byref(self._st),
+                                           C.byref(spec), C.byref(rspec), None if m is None else m.data_ptr(),
+                                           out.data_ptr(), self.dev_index, self._stream()))
+
     def env_reward(self, spec: abi.SgEnvSpec, reward: torch.Tensor, terms: torch.Tensor,
                    terminated: torch.Tensor, truncated: torch.Tensor) -> None:
         """sg_env_reward into preallocated reward (fp32 [N, A]), terms (fp32 [N, A, 5]) and flags (uint8 [N])."""

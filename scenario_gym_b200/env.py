@@ -39,7 +39,11 @@ class ObsSpec:
     distance to the first box of another present entity, at most ``lidar_range`` metres.  With ``map_edges`` = Km
     (0..32) it also sees the Km road-network edges (of the driveable, walkable and impenetrable surfaces) nearest to
     it within ``map_radius`` metres: the nearest point and both end points in its frame, which surfaces the edge
-    bounds, and a valid flag (10 floats each, between the road block and the lidar)."""
+    bounds, and a valid flag (10 floats each, between the road block and the lidar).  With ``raster_size`` = S
+    (0, or a multiple of 32 in 32..256) each agent also gets a bird's-eye raster, uint8 [5, S, S] of 0 / 1 in
+    ``info["raster"]``, kept out of the observation rows: ``raster_resolution`` metres per pixel, centred
+    ``raster_ahead`` metres ahead of the agent, row 0 ahead and column 0 to the left, with channels
+    ``VecScenarioEnv.raster_channels`` (include/sg_b200.h, SgRasterSpec)."""
     k_neighbours: int = 8
     radius: float = 50.0
     lookahead: Sequence[float] = (1.0, 2.0, 3.0)
@@ -48,6 +52,9 @@ class ObsSpec:
     lidar_range: float = 50.0
     map_edges: int = 0
     map_radius: float = 50.0
+    raster_size: int = 0
+    raster_resolution: float = 0.5
+    raster_ahead: float = 0.0
 
     @property
     def n_features(self) -> int:
@@ -109,6 +116,10 @@ class VecScenarioEnv:
     with the agents' starts perturbed (``sg_reset_scenarios_init``); ``start_window`` [N] fp64 holds the longest
     delay after t0 each scenario allows (every vehicle of the log still present, ``min_remaining`` seconds left).
     A pedestrian starting later restarts at the first point of its route, as at t0: routes are not re-targeted.
+
+    With ``ObsSpec(raster_size=S)`` every agent also gets a bird's-eye raster (``sg_env_raster``): ``reset()`` and
+    ``step()`` return ``info["raster"]`` uint8 [N, A, 5, S, S] (channels ``raster_channels``), and ``step()``
+    ``info["final_raster"]``, the raster of the state each scenario ended the step in, before its reset.
     """
 
     def __init__(self, scenarios: List[Scenario], create_agent: Callable = _ego_policy,
@@ -140,6 +151,15 @@ class VecScenarioEnv:
             raise ValueError(f"ObsSpec: map_edges must be in 0..32, got {self.obs_spec.map_edges}")
         if Km > 0 and not (math.isfinite(float(self.obs_spec.map_radius)) and float(self.obs_spec.map_radius) > 0):
             raise ValueError(f"ObsSpec: map_radius must be finite and > 0, got {self.obs_spec.map_radius}")
+        S = self.obs_spec.raster_size
+        if isinstance(S, bool) or int(S) != S or not (S == 0 or (32 <= S <= 256 and int(S) % 32 == 0)):
+            raise ValueError(f"ObsSpec: raster_size must be 0 or a multiple of 32 in 32..256, got {S}")
+        S = int(S)
+        if S > 0 and not (math.isfinite(float(self.obs_spec.raster_resolution))
+                          and float(self.obs_spec.raster_resolution) > 0):
+            raise ValueError(f"ObsSpec: raster_resolution must be finite and > 0, got {self.obs_spec.raster_resolution}")
+        if S > 0 and not math.isfinite(float(self.obs_spec.raster_ahead)):
+            raise ValueError(f"ObsSpec: raster_ahead must be finite, got {self.obs_spec.raster_ahead}")
         w = dict(DEFAULT_REWARD_WEIGHTS)
         if isinstance(reward_weights, Mapping):
             unknown = set(reward_weights) - set(abi.ENV_TERMS)
@@ -229,6 +249,23 @@ class VecScenarioEnv:
         self._spec = spec
         self._info = {"agent_mask": self._agent_mask, "episode_step": eng.tensor("tick"), "episode": self._episode}
 
+        # the raster (sg_env_raster): its buffers and the polygons' bounding boxes, built once
+        self.raster_channels = abi.RASTER_CHANNELS
+        self._raster = self._final_raster = None
+        if S > 0:
+            sc = eng.scene
+            rspec = abi.SgRasterSpec()
+            rspec.size, rspec.n_networks = S, sc.n_networks
+            rspec.resolution, rspec.ahead = float(self.obs_spec.raster_resolution), float(self.obs_spec.raster_ahead)
+            box, rspec.margin = abi.raster_poly_boxes(sc.rn_edge_off, sc.rn_edges,
+                                                      abi.raster_half_diagonal(S, rspec.resolution))
+            self._poly_box = torch.from_numpy(box if len(box) else np.zeros((1, 4))).to(dev)
+            rspec.poly_box = self._poly_box.data_ptr()
+            self._rspec = rspec
+            self._raster = zeros(N, self.A, 5, S, S, dtype=torch.uint8)
+            self._final_raster = zeros(N, self.A, 5, S, S, dtype=torch.uint8)
+            self._info["raster"] = self._raster
+
         # episode starts (sg_reset_scenarios_init): the valid windows are decided once, on the host
         self.reset_spec = reset_spec
         rs = reset_spec if reset_spec is not None else ResetSpec()
@@ -306,6 +343,8 @@ class VecScenarioEnv:
         self._episode.zero_()
         self._resets += 1  # (a planner cannot see this reset in the episode counters when they were 0)
         eng.env_observe(self._spec, self._obs, self._agent_mask)
+        if self._raster is not None:
+            eng.env_raster(self._spec, self._rspec, self._raster)
         return self._obs, dict(self._info)
 
     def step(self, actions: torch.Tensor):
@@ -329,6 +368,9 @@ class VecScenarioEnv:
         eng.env_reward(self._spec, self._reward, self._terms, self._terminated, self._truncated)
         eng.env_observe(self._spec, self._obs, self._agent_mask)
         self._final_obs.copy_(self._obs)
+        if self._raster is not None:
+            eng.env_raster(self._spec, self._rspec, self._raster)
+            self._final_raster.copy_(self._raster)
         for k, f in _FINAL_FIELDS.items():
             self._final[k].copy_(eng.tensor(f))
         torch.bitwise_or(self._terminated, self._truncated, out=self._finished)
@@ -338,9 +380,13 @@ class VecScenarioEnv:
             eng.reset(mask=self._finished, init=self._init)
             self._counter.add_(self._finished)
         eng.env_observe(self._spec, self._obs, self._agent_mask, mask=self._finished)
+        if self._raster is not None:
+            eng.env_raster(self._spec, self._rspec, self._raster, mask=self._finished)
         self._episode.add_(self._finished)
         eng.tensor("event_count").zero_()  # ego collision events are not kept across steps
         info = dict(self._info, final_obs=self._final_obs, final=self._final, terms=self._terms)
+        if self._raster is not None:
+            info["final_raster"] = self._final_raster
         return self._obs, self._reward, self._terminated.view(torch.bool), self._truncated.view(torch.bool), info
 
 

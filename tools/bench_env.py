@@ -3,7 +3,7 @@
 bench_env.py -- throughput of the closed-loop environment (VecScenarioEnv) and where its step goes.
 
     python tools/bench_env.py [--out FILE] [--lidar R] [--map Km] [--reset]   # one JSON line per workload on
-                                                                               # stdout (and appended to FILE)
+                              [--raster S [--raster-brute LIB]]               # stdout (and appended to FILE)
 
 Workloads:
   vehicles  12 500 scenarios x 64 VehicleController entities (synthetic.vehicles_config, 625 distinct
@@ -14,7 +14,8 @@ Observation: K = 8 neighbours within 50 m, lookahead 1 / 2 / 3 s, and with --lid
 reaching 50 m (ObsSpec.lidar_rays; 0, the default, leaves the workloads as they were).  With --map Km > 0 every
 scenario drives over a synthetic town (synthetic.grid_town: the vehicles' 400 m square, or one town over the 23 test
 scenes' trajectory points, 0.5 .. 99.5 % range) and observes its Km nearest road-network edges within 50 m (ObsSpec.map_edges; 0, the default, attaches no
-town and leaves the workloads as they were).  The policy is a trivial
+town and leaves the workloads as they were).  --raster S > 0 attaches the same town and gives every agent a bird's-eye
+raster of S x S pixels of 0.5 m (ObsSpec.raster_size).  The policy is a trivial
 torch function of the observation (steer toward the first lookahead point).  SG_B200_LIB selects the library
 (e.g. a variant built by tools/build_variant.sh); `library` in the record names it.
 
@@ -36,6 +37,13 @@ Reported per workload:
                                         (sg_reset_scenarios) and the init kernel (sg_reset_scenarios_init)
   env_steps_per_s_spec / _plain         with --reset: step() + policy with the spec's auto-reset, and with the plain
                                         one (env.reset_spec = None), host clock over >= 1 s each
+  raster_size / raster_bytes            with --raster: S and the bytes one sg_env_raster call writes (N*A*5*S*S)
+  raster_us / raster_TBps / raster_floor_us   its device time per call (CUDA events over 20 calls, every scenario),
+                                        the write rate, and the time the bytes take at 7.7 TB/s
+  raster_brute_us                       with --raster-brute LIB: the same call through LIB, a library built with
+                                        -DSG_RASTER_BRUTE (tools/build_variant.sh), on the same buffers
+  env_steps_per_s_raster / _no_raster   with --raster: step() + policy with the raster, and without it (the same env
+                                        with its raster switched off), host clock over >= 1 s each
   device / power_limit_w                the card and its power limit
 """
 from __future__ import annotations
@@ -76,7 +84,7 @@ def vehicles_env(obs, reset_spec=None):
     cfg = synthetic.vehicles_config(seed=0, N=distinct, M=M, T=256)
     rows = synthetic.two_knot_rows(cfg).reshape(distinct, M, 2, 7)
     ce = CatalogEntry(None, "car1", "car", "Vehicle", BoundingBox(*synthetic.CAR1_BOX))
-    town = synthetic.grid_town(seed=0, half_extent=200.0) if obs.map_edges > 0 else None
+    town = synthetic.grid_town(seed=0, half_extent=200.0) if obs.map_edges > 0 or obs.raster_size > 0 else None
     scs = [Scenario([Vehicle(ce, trajectory=Trajectory(rows[n, m]), ref="ego" if m == 0 else f"entity_{m}")
                      for m in range(M)], road_network=town) for n in range(distinct)]
     return VecScenarioEnv(scs * reps, create_agent=lambda s, e: PolicyAgent(e), timestep=cfg.dt, obs=obs,
@@ -98,7 +106,7 @@ def xosc_env(obs, reset_spec=None):
             ce = CatalogEntry(None, "entry", None, ctype, BoundingBox(*[float(v) for v in inp["box"][i]]))
             ents.append(C(ce, trajectory=Trajectory(inp[f"traj{i}"]), ref=man[name]["refs"][i]))
         scs.append(Scenario(ents))
-    if obs.map_edges > 0:  # one town over the test scenes: the 0.5 .. 99.5 % range of their trajectory points
+    if obs.map_edges > 0 or obs.raster_size > 0:  # one town over the test scenes: the 0.5 .. 99.5 % range of their trajectory points
         # (one scene has a stray point thousands of km away, which a town cannot sensibly cover)
         xy = np.concatenate([np.asarray(e.trajectory.data)[:, 1:3] for sc in scs for e in sc.entities])
         lo, hi = np.quantile(xy, 0.005, axis=0), np.quantile(xy, 0.995, axis=0)
@@ -119,7 +127,7 @@ def card():
     return name, power
 
 
-def measure(name, env):
+def measure(name, env, brute_lib=None):
     eng = env._engine
     stream = torch.cuda.current_stream()
     o, _ = env.reset()
@@ -192,6 +200,7 @@ def measure(name, env):
     del fused
     maps = map_times(env) if env.obs_spec.map_edges > 0 else {}
     resets = reset_times(env) if env.reset_spec is not None else {}
+    rasters = raster_times(env, brute_lib) if env.obs_spec.raster_size > 0 else {}
     F = env.n_features
     obs_bytes = env.N * env.A * (4 * F + 1 + 9) + env.N * 9
     dev, power = card()
@@ -206,7 +215,7 @@ def measure(name, env):
         "observe_bytes": obs_bytes, "observe_GBps": obs_bytes / (acc["observe"] * 1e-6) / 1e9,
         "lidar_rays": int(env.obs_spec.lidar_rays), "lidar_bytes": env.N * env.A * 4 * int(env.obs_spec.lidar_rays),
         "map_edges": int(env.obs_spec.map_edges), "map_bytes": env.N * env.A * 40 * int(env.obs_spec.map_edges),
-        **maps, **resets,
+        **maps, **resets, **rasters,
         "library": os.path.basename(abi.PRODUCT_LIB),
         "device": dev, "power_limit_w": power,
     }
@@ -240,6 +249,52 @@ def map_times(env):
     return {"map_table_edges": int(env._map["map_off"][-1].item()), "map_grid_cells": int((dims[:, 0] * dims[:, 1]).sum()),
             "map_cell_m": float(env._map["map_grid"][0, 2].item()), "observe_no_map_us": round(base, 2),
             "map_us": round(grid - base, 2), "map_brute_us": round(flat - base, 2)}
+
+
+def raster_times(env, brute_lib=None):
+    """sg_env_raster's device time per call (every scenario), through the product and, given a library built with
+    -DSG_RASTER_BRUTE, through it on the same buffers; the env's steps per second with and without its raster."""
+    import ctypes as C
+
+    eng, stream = env._engine, torch.cuda.current_stream()
+    S = int(env.obs_spec.raster_size)
+
+    def raster_us(call, reps):
+        for _ in range(2):
+            call()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record(stream)
+        for _ in range(reps):
+            call()
+        e1.record(stream)
+        torch.cuda.synchronize()
+        return e0.elapsed_time(e1) * 1e3 / reps
+
+    nbytes = env._raster.numel()
+    out = {"raster_size": S, "raster_resolution": float(env.obs_spec.raster_resolution), "raster_bytes": nbytes,
+           "raster_polygons": int(len(eng.scene.rn_edge_off) - 1)}
+    us = raster_us(lambda: eng.env_raster(env._spec, env._rspec, env._raster), 20)
+    out.update(raster_us=round(us, 2), raster_TBps=round(nbytes / (us * 1e-6) / 1e12, 3),
+               raster_floor_us=round(nbytes / 7.7e12 * 1e6, 2))
+    if brute_lib:
+        lib = abi.bind(C.CDLL(os.path.abspath(brute_lib)), "sg_")
+        want = env._raster.clone()
+
+        def brute():
+            rc = lib["env_raster"](C.byref(eng._sc), C.byref(eng.params), C.byref(eng._st), C.byref(env._spec),
+                                   C.byref(env._rspec), None, env._raster.data_ptr(), eng.dev_index, eng._stream())
+            if rc:
+                raise RuntimeError(lib["last_error"]().decode())
+
+        out["raster_brute_us"] = round(raster_us(brute, 3), 2)
+        out["raster_brute_equal"] = bool(torch.equal(want, env._raster))
+        out["raster_brute_library"] = os.path.basename(brute_lib)
+        del want
+    out["env_steps_per_s_raster"] = steps_per_s(env)
+    keep, env._raster = env._raster, None  # (step() skips the raster)
+    out["env_steps_per_s_no_raster"] = steps_per_s(env)
+    env._raster = keep
+    return out
 
 
 def steps_per_s(env):
@@ -298,16 +353,18 @@ def main():
     ap.add_argument("--lidar", type=int, default=0, help="lidar rays R of the observation (0: no lidar block)")
     ap.add_argument("--map", type=int, default=0, help="map edges Km of the observation (0: no town, no map block)")
     ap.add_argument("--reset", action="store_true", help="build the envs with RESET_SPEC and time the resets")
+    ap.add_argument("--raster", type=int, default=0, help="raster size S (0: no town, no raster)")
+    ap.add_argument("--raster-brute", default=None, help="a library built with -DSG_RASTER_BRUTE to time as well")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("bench_env.py measures the GPU engine: no CUDA device")
     obs = ObsSpec(k_neighbours=8, radius=50.0, lookahead=(1.0, 2.0, 3.0), lidar_rays=args.lidar, lidar_range=50.0,
-                  map_edges=args.map, map_radius=50.0)
+                  map_edges=args.map, map_radius=50.0, raster_size=args.raster, raster_resolution=0.5)
     for w in args.workloads.split(","):
         t0 = time.time()
         env = {"vehicles": vehicles_env, "xosc": xosc_env}[w](obs, RESET_SPEC if args.reset else None)
         build_s = time.time() - t0
-        rec = measure(w, env)
+        rec = measure(w, env, args.raster_brute)
         rec["build_s"] = round(build_s, 1)
         line = json.dumps(rec)
         print(line, flush=True)
